@@ -6,6 +6,7 @@ screen-tile sharded over N GPUs (strong scaling: the frame is fixed, the tiles a
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own CPU tracer (oracle/_ref) on the host cores
+    python bench.py --dump-outputs DIR ...    # also writes what the last timed step computed (dump_outputs) as DIR/*.npy
 
 A step is one full frame.  `value` = rays of the whole frame / device time (CUDA events on the launching stream, scene
 and all buffers resident in HBM, max over ranks); `e2e` = the same frame through the public call with a HOST
@@ -74,6 +75,29 @@ def emit(obj):
     out = _JSON_OUT or sys.stdout
     out.write(json.dumps(obj) + "\n")
     out.flush()
+
+
+# 24 B per dumped pixel (16 B of float32 channels in frame.npy + an 8 B float64 index in frame_pixels.npy): 48 MiB at most
+DUMP_PIXELS = 1 << 21
+RAY_COUNTERS = ("primary_rays", "shadow_rays", "reflection_rays", "reflection_shadow_rays", "primary_hits")
+
+
+def dump_outputs(out_dir, argb, counts):
+    """What the timed path handed its caller in the last timed step, for comparing two builds output for output (the
+    inputs of a workload are seeded, so they are the same from run to run):
+      frame.npy        [n, 4] float32: the A, R, G, B bytes of the ARGB32 frame at the pixels of frame_pixels.npy
+      frame_pixels.npy [n] float64: their row-major indices -- every pixel, or a fixed seeded sample of DUMP_PIXELS of them
+      ray_counts.npy   [5] float64: the step's RAY_COUNTERS summed over the ranks (the whole frame at any GPU count)"""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    argb = np.ascontiguousarray(argb).view(np.uint32).reshape(-1)
+    idx = np.arange(argb.size)
+    if argb.size > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(argb.size, DUMP_PIXELS, replace=False))
+    px = argb[idx]
+    np.save(out / "frame.npy", np.stack([(px >> np.uint32(s)) & np.uint32(0xff) for s in (24, 16, 8, 0)], -1).astype(np.float32))
+    np.save(out / "frame_pixels.npy", idx.astype(np.float64))
+    np.save(out / "ray_counts.npy", np.float64(counts))
 
 
 def make_scene(name):
@@ -377,6 +401,10 @@ def run_ours(args, scene):
         sync_all()
         assert len(done) == args.steps
         st = done[-1]
+        # --dump-outputs: a device copy of the last timed frame (its buffer is rendered into again below); it goes to the
+        # host and to disk only after every measurement
+        last_frame = frames[(pipe.next - 1) % len(frames)].frame.clone() if args.dump_outputs and rank == 0 else None
+        last_counts = [getattr(st, k) for k in RAY_COUNTERS]
         launches = sum(d.kernel_launches + (2 if frame.mode == "nccl" else 0) for d in done)   # + the pack and unpack kernels of the nccl-mode gather
         dev_ms = ev0.elapsed_time(ev1)
         rays_rank, traced_rank = st.total_rays, st.traced_rays
@@ -464,6 +492,10 @@ def run_ours(args, scene):
     rays_total = reduce(float(rays_rank), dist.ReduceOp.SUM if world > 1 else None)
     traced_total = reduce(float(traced_rank), dist.ReduceOp.SUM if world > 1 else None)
     launches_total = reduce(float(launches), dist.ReduceOp.SUM if world > 1 else None)
+    if args.dump_outputs:
+        counts = [reduce(float(c), dist.ReduceOp.SUM if world > 1 else None) for c in last_counts]
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last_frame.cpu().numpy(), counts)
     ms_step = dev_ms / args.steps
     value = rays_total / ms_step / 1e3
 
@@ -576,7 +608,13 @@ def main():
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"], help="N > 1: how the frame gets to rank 0 (raytracercpp_b200/distributed.py)")
     ap.add_argument("--lib", default=None, help="another build of librtb200 (kernel A/B experiments)")
     ap.add_argument("--leaf-split", type=int, default=None, help="RT_OPT_LEAF_SPLIT override (experiments); default = library default")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame and ray counters of the last timed step as DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     claim_stdout()
     if args.tile is None:
         args.tile = 64 if int(os.environ.get("WORLD_SIZE", 1)) == 1 else 32

@@ -1,5 +1,5 @@
 // Compiles include/rtb200_renderer.hpp against the REAL value types of the reference (triangle.h, materials.h, image.h,
-// mat.h, vec.h, included from /root/reference/tp2 where they lie -- nothing is copied) and instantiates every templated
+// mat.h, vec.h, included from the original's tp2 directory, RTB200_REFERENCE, where they lie -- nothing is copied) and instantiates every templated
 // member with them: the duck-typing the adapter relies on is checked against the reference's own declarations, not
 // against stand-in structs.  CPU-only translation unit; built as an object file by tests/test_abi.py (no GPU, not run).
 #include <vector>

@@ -7,6 +7,7 @@ logic, the ABI surface of the CUDA library, and the kernels' per-ray source comp
 from __future__ import annotations
 
 import ctypes
+import os
 import subprocess
 import sys
 from pathlib import Path
@@ -18,6 +19,17 @@ ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 
 GOLDEN = ROOT / "tests" / "golden"
+# The original RayTracerCPP sources (its tp2 directory) are not part of this repository.  The live comparisons with them
+# run where RTB200_REFERENCE names that directory (`make -C oracle ref` compiles it into oracle/_ref) and skip elsewhere;
+# the committed goldens under tests/golden carry what they were compared against.
+REFERENCE = Path(os.environ["RTB200_REFERENCE"]) if os.environ.get("RTB200_REFERENCE") else None
+
+
+def require_reference() -> Path:
+    """For the golden generators (tests/golden/make_golden*.py): the original's tp2 directory, or a clear stop."""
+    if REFERENCE is None or not REFERENCE.is_dir():
+        raise SystemExit("the original sources are needed: export RTB200_REFERENCE=<RayTracerCPP>/tp2, then make -C oracle ref")
+    return REFERENCE
 
 
 def pytest_configure(config):
@@ -48,7 +60,7 @@ def oracle():
 def ref_strict():
     from oracle import bindings
     if not bindings.available("ref_strict"):
-        pytest.skip("oracle/_ref/libref_strict.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libref_strict.so not built (needs the original sources, RTB200_REFERENCE)")
     return bindings.CpuTracer("ref_strict")
 
 
@@ -56,7 +68,7 @@ def ref_strict():
 def ref_fma():
     from oracle import bindings
     if not bindings.available("ref"):
-        pytest.skip("oracle/_ref/libref.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libref.so not built (needs the original sources, RTB200_REFERENCE)")
     return bindings.CpuTracer("ref")
 
 

@@ -1,8 +1,9 @@
 """Cuts the golden fixtures of tests/golden/ from the UNMODIFIED reference compiled in this container
 (oracle/_ref/libref_strict.so = reference sources with -ffp-contract=off, oracle/_ref/libref.so = reference flags).
 
-Run here (needs /root/reference):   python tests/golden/make_golden.py
-The .npz files are committed; the GPU box has no /root/reference and only reads them.
+Run where the original sources are (export RTB200_REFERENCE=<RayTracerCPP>/tp2; make -C oracle ref):
+    python tests/golden/make_golden.py
+The .npz files are committed; the tests only read them.
 
 Contents
   robot_scene.npz    robot.obj through the reference's own loader (read_meshio_data + MeshIOUtils::create_triangles,
@@ -25,6 +26,7 @@ sys.path.insert(0, str(ROOT))
 from oracle.bindings import CpuTracer, default_settings  # noqa: E402
 from raytracercpp_b200 import scenes  # noqa: E402
 from raytracercpp_b200.renderer import precompute_materials  # noqa: E402
+from tests.conftest import require_reference  # noqa: E402
 
 OUT = Path(__file__).resolve().parent
 MAT_KEYS = ("ambient_coeff", "diffuse", "specular", "emission")
@@ -106,10 +108,11 @@ def render_with(tracer, scene, kw, mats, tex, fov=80.0, seeded=False):
 
 
 def main():
+    ref = require_reference()
     strict, fma = CpuTracer("ref_strict"), CpuTracer("ref")
     T = np.eye(4, dtype=np.float32)
     T[1, 3], T[2, 3] = -2, -4
-    xyz9, uv6, mat, mats = strict.load_obj("/root/reference/tp2/data/Robot/robot.obj", T)
+    xyz9, uv6, mat, mats = strict.load_obj(str(ref / "data" / "Robot" / "robot.obj"), T)
     mats = precompute_materials(mats)
     np.savez_compressed(OUT / "robot_scene.npz", xyz9=xyz9, uv6=uv6, mat=mat, materials=mats_to_rows(mats))
     scene = dict(xyz9=xyz9, uv6=uv6, mat=mat)

@@ -1,7 +1,7 @@
 """Cuts tests/golden/golden_fullsize.npz: BASELINE.json's configs at their FULL sizes, from the UNMODIFIED reference
 compiled in this container (oracle/_ref/libref_strict.so; libref.so = the reference's own FMA flags for the CRCs).
 
-    python tests/golden/make_golden_fullsize.py        (needs /root/reference; ~2 minutes)
+    python tests/golden/make_golden_fullsize.py        (needs the original sources: RTB200_REFERENCE, see make_golden.py; ~2 minutes)
 
 Per frame: the CRC32 of the whole ARGB32 image (pins the oracle bit-exactly on the CPU side), every FULL_ROW_STEP-th
 row (what the GPU frame is compared with, within the north-star tolerance), and the ray counts.
@@ -23,6 +23,7 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 
 from oracle.bindings import CpuTracer  # noqa: E402
+from tests.conftest import require_reference  # noqa: E402
 from raytracercpp_b200 import scenes  # noqa: E402
 from raytracercpp_b200.renderer import precompute_materials  # noqa: E402
 from tests import common  # noqa: E402
@@ -35,6 +36,7 @@ def crc(img):
 
 
 def main():
+    require_reference()
     strict, fma = CpuTracer("ref_strict"), CpuTracer("ref")
     z = np.load(OUT / "robot_scene.npz")
     rows = z["materials"]

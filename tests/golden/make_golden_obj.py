@@ -3,7 +3,7 @@ tp2/src/mesh_io.cpp:426-591, tp2/projets/utils/meshIOUtils.cpp:4-33; compiled in
 fixture files under tests/golden/obj/ -- triangles, texture coordinates, material indices, material table -- for the
 parity test of csrc/scene_io.cpp (tests/test_scene_io.py).
 
-    python tests/golden/make_golden_obj.py        (needs /root/reference)
+    python tests/golden/make_golden_obj.py        (needs the original sources: RTB200_REFERENCE, see make_golden.py)
 """
 from __future__ import annotations
 
@@ -16,6 +16,7 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 
 from oracle.bindings import CpuTracer  # noqa: E402
+from tests.conftest import require_reference  # noqa: E402
 
 OUT = Path(__file__).resolve().parent
 TRANSFORM = np.float32([[0.5, 0, 0, 0.25], [0, 2.0, 0, -2.0], [0, 0, 1.0, -4.0], [0, 0, 0, 1]])
@@ -27,6 +28,7 @@ def rows(mats):
 
 
 def main():
+    require_reference()
     strict = CpuTracer("ref_strict")
     out = {"transform": TRANSFORM}
     for name, tr in (("fixture_uv", TRANSFORM), ("fixture_plain", None)):

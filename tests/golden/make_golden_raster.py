@@ -3,7 +3,7 @@ renderer.cpp:869-1006) from the UNMODIFIED reference compiled in this container 
 thread -- raster_trace() walks the triangles under `omp parallel for` over an unsynchronised z-buffer, so the sequential
 order is the reproducible one -- and, for the SSAO case, after srand(RASTER_SRAND) as in make_golden_ssao.py.
 
-    python tests/golden/make_golden_raster.py        (needs /root/reference)
+    python tests/golden/make_golden_raster.py        (needs the original sources: RTB200_REFERENCE, see make_golden.py)
 
 Per set-up of tests/common.py::raster_table that has no rough reflections: the reference's frame (and the nine SSAO
 generator seeds where SSAO is on).  The oracle must reproduce every frame bit for bit before the file is written.
@@ -19,12 +19,14 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 
 from oracle.bindings import CpuTracer  # noqa: E402
+from tests.conftest import require_reference  # noqa: E402
 from tests import common  # noqa: E402
 
 OUT = Path(__file__).resolve().parent
 
 
 def main():
+    require_reference()
     strict, orc = CpuTracer("ref_strict"), CpuTracer("oracle")
     z = np.load(OUT / "robot_scene.npz")
     mats = [dict(ambient_coeff=tuple(r[0:3]), diffuse=tuple(r[3:6]), specular=tuple(r[6:9]), emission=tuple(r[9:12]),

@@ -2,7 +2,7 @@
 container (oracle/_ref/libref_strict.so), its SSAO pass run on one thread after srand(SRAND_SEED) -- the only reproducible
 way to run it: its generators are seeded from std::rand() and the OpenMP thread number.
 
-    python tests/golden/make_golden_ssao.py        (needs /root/reference)
+    python tests/golden/make_golden_ssao.py        (needs the original sources: RTB200_REFERENCE, see make_golden.py)
 
 Per set-up of tests/common.py::ssao_table: the reference's frame, the nine generator seeds that run used (lanes 0..7 of the
 8-lane generator, the scalar generator), and the oracle's frame with the per-pixel stream the CUDA path shares.
@@ -18,6 +18,7 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 
 from oracle.bindings import CpuTracer  # noqa: E402
+from tests.conftest import require_reference  # noqa: E402
 from tests import common  # noqa: E402
 
 OUT = Path(__file__).resolve().parent
@@ -25,6 +26,7 @@ SRAND_SEED = 20261019
 
 
 def main():
+    require_reference()
     strict, orc = CpuTracer("ref_strict"), CpuTracer("oracle")
     z = np.load(OUT / "robot_scene.npz")
     mats = [dict(ambient_coeff=tuple(r[0:3]), diffuse=tuple(r[3:6]), specular=tuple(r[6:9]), emission=tuple(r[9:12]),

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from raytracercpp_b200 import api, build
-from tests.conftest import cuda_available
+from tests.conftest import REFERENCE, cuda_available
 
 ROOT = Path(__file__).resolve().parents[1]
 
@@ -80,12 +80,12 @@ def test_tile_ownership_is_a_partition(lib):
 
 def test_adapter_compiles_against_the_reference_headers(tmp_path):
     """include/rtb200_renderer.hpp with the reference's REAL Triangle / Materials / Image / Transform / Point / Vector
-    (headers included from /root/reference/tp2 where they lie; Qt's QImage from the oracle's shim): every templated
-    member is instantiated with them.  CPU-only object file; needs the mounted reference (this container)."""
+    (headers included from the original sources where they lie; Qt's QImage from the oracle's shim): every templated
+    member is instantiated with them.  CPU-only object file; needs the original sources (RTB200_REFERENCE)."""
     import subprocess
-    ref = Path("/root/reference/tp2")
-    if not (ref / "projets" / "triangle.h").exists():
-        pytest.skip("/root/reference is not mounted here")
+    ref = REFERENCE
+    if ref is None or not (ref / "projets" / "triangle.h").exists():
+        pytest.skip("the original sources are not here (RTB200_REFERENCE)")
     obj = tmp_path / "adapter_reference_types.o"
     inc = [ROOT / "include", ROOT / "oracle" / "qt_shim", ref / "src", ref / "projets", ref / "projets" / "utils", ref / "projets" / "renderer",
            ref / "projets" / "scene"]

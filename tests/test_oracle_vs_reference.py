@@ -1,5 +1,5 @@
-"""The oracle against the compiled reference itself (oracle/_ref), live: skipped where /root/reference was never
-available to build it.  Pins, among others, the argument evaluation order of renderer.cpp:313."""
+"""The oracle against the compiled reference itself (oracle/_ref), live: skipped unless RTB200_REFERENCE named the
+original sources when oracle/_ref was built (tests/conftest.py).  Pins, among others, the argument evaluation order of renderer.cpp:313."""
 import numpy as np
 import pytest
 

@@ -9,9 +9,17 @@ import pytest
 
 from raytracercpp_b200 import api
 from raytracercpp_b200.renderer import precompute_materials
+from tests.conftest import REFERENCE
 
 GOLDEN = Path(__file__).resolve().parent / "golden"
-REF_DATA = Path("/root/reference/tp2/data")
+REF_DATA = REFERENCE / "data" if REFERENCE is not None else None
+
+
+def reference_file(rel):
+    path = REF_DATA / rel if REF_DATA is not None else None
+    if path is None or not path.exists():
+        pytest.skip("reference data not here (RTB200_REFERENCE)")
+    return path
 
 
 @pytest.fixture(scope="module")
@@ -61,9 +69,7 @@ def test_material_offset_and_errors(lib, tmp_path):
 def test_robot_scene_fixture_is_what_the_loader_gives(lib, robot):
     """tests/golden/robot_scene.npz was cut with the reference's loader from its robot.obj at the GUI's placement,
     Translation(0, -2, -4) (QT/mainwindow.cpp:308-312); where that file is mounted the native loader must give the same."""
-    path = REF_DATA / "Robot" / "robot.obj"
-    if not path.exists():
-        pytest.skip("reference data not mounted")
+    path = reference_file("Robot/robot.obj")
     tr = np.float32([[1, 0, 0, 0], [0, 1, 0, -2], [0, 0, 1, -4], [0, 0, 0, 1]])
     xyz9, uv6, mat, mats, names = api.load_obj(path, tr, lib=lib)
     assert np.array_equal(xyz9, robot["xyz9"]) and np.array_equal(uv6, robot["uv6"]) and np.array_equal(mat, robot["mat"])
@@ -77,9 +83,7 @@ def test_robot_scene_fixture_is_what_the_loader_gives(lib, robot):
 
 @pytest.mark.parametrize("rel", ["Robot/robot.obj", "Geometry/geometry.obj", "cube.obj"])
 def test_reference_data_live(lib, ref_strict, rel):
-    path = REF_DATA / rel
-    if not path.exists():
-        pytest.skip("reference data not mounted")
+    path = reference_file(rel)
     tr = np.float32([[0.02, 0, 0, -1], [0, 0.02, 0, -3], [0, 0, 0.02, -13], [0, 0, 0, 1]])
     xyz9, uv6, mat, mats, _ = api.load_obj(path, tr, lib=lib)
     rx, ruv, rmat, rmats = ref_strict.load_obj(str(path), tr)
