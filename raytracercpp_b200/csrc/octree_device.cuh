@@ -599,6 +599,104 @@ __global__ void k_ob_top_table(float4* recs, float4* top, Stats* st)
     st->top_n = (unsigned int)used;
 }
 
+// ---- wrecs[]: the wide copy of the tree that the packet kernels traverse.  A packet's cell round (pop, fetch, stage,
+// pyramid cull, slab tests, insertion) has a fixed cost sized for 8 children, and a cell of the reference's octree has 2.6
+// on average (10 M-triangle sphere): one round per level.  Every block of wrecs[] is a collapse of the tree below one owner
+// record instead.  Collapse rule: the block starts as the owner's children; repeatedly, the interior member with the
+// largest surface area of its axis box (first three slabs) among those whose children still fit (members - 1 + its count
+// <= 8) is replaced IN PLACE by its children, ties to the lower position; it stops when no member fits.  Members spliced in
+// can be absorbed in turn, so a block may reach several levels down.
+// A node of the wide tree is a record of recs[] (`src`): leaves are copied unchanged (same triangles), interior records
+// get their wide block and member count.  Same pattern as the narrow build: nodes frontier by frontier (k_wb_collapse,
+// scan, k_wb_children), sizes bottom-up (k_wb_size), positions top-down (k_ob_place), then the records (k_wb_records).
+// The nodes on a root-to-leaf path of wrecs[] are a subset of those of the same path in recs[], so the wide tree is never
+// deeper and the packet stack bound of the narrow tree holds.
+__device__ __forceinline__ bool wb_interior(uint32_t meta) { return !(meta & RT_META_LEAF) && (meta & RT_META_COUNT_MASK) != 0u; }
+
+__device__ __forceinline__ float wb_axis_area(const float4* recs, uint32_t r)      // half the surface area of the axis box
+{
+    const float4 q0 = recs[4 * (size_t)r], q1 = recs[4 * (size_t)r + 1];
+    const float dx = q0.y - q0.x, dy = q0.w - q0.z, dz = q1.y - q1.x;
+    return dx * dy + dy * dz + dz * dx;
+}
+
+// members[8 j ..] = the block of node lf + j (a record of recs[] that is interior), counts[j] = its size (0: leaf)
+__global__ void __launch_bounds__(256)
+k_wb_collapse(const float4* recs, const uint32_t* src, uint32_t lf, uint32_t lc, uint32_t* info, uint32_t* counts, uint32_t* members)
+{
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= lc) return;
+    const float4 own = recs[4 * (size_t)src[lf + j] + 3];
+    const uint32_t meta = __float_as_uint(own.w);
+    if (!wb_interior(meta)) { counts[j] = 0u; info[lf + j] = 0u; return; }
+    uint32_t m[8], kids[8], link[8];
+    float area[8];
+    int n = 0;
+    auto put = [&](int at, uint32_t r) {
+        const float4 q3 = recs[4 * (size_t)r + 3];
+        const uint32_t mm = __float_as_uint(q3.w);
+        m[at] = r;
+        kids[at] = wb_interior(mm) ? (mm & RT_META_COUNT_MASK) : 0u;
+        link[at] = __float_as_uint(q3.z);
+        area[at] = kids[at] ? wb_axis_area(recs, r) : 0.0f;
+    };
+    const uint32_t first = __float_as_uint(own.z), count = meta & RT_META_COUNT_MASK;
+    for (uint32_t k = 0; k < count; k++) put(n++, first + k);
+    for (;;) {
+        int best = -1;
+        for (int k = 0; k < n; k++)
+            if (kids[k] && n - 1 + (int)kids[k] <= 8 && (best < 0 || area[k] > area[best])) best = k;
+        if (best < 0) break;
+        const int c = (int)kids[best];
+        const uint32_t l = link[best];
+        for (int k = n - 1; k > best; k--) {                                   // the members behind it move c - 1 places up
+            m[k + c - 1] = m[k]; kids[k + c - 1] = kids[k]; link[k + c - 1] = link[k]; area[k + c - 1] = area[k];
+        }
+        for (int k = 0; k < c; k++) put(best + k, l + (uint32_t)k);
+        n += c - 1;
+    }
+    for (int k = 0; k < n; k++) members[8 * (size_t)j + k] = m[k];
+    counts[j] = (uint32_t)n;
+    info[lf + j] = (uint32_t)n | (kCellRefInterior << 4);
+}
+
+// the members of the frontier's blocks become the next frontier; counts[] now holds the exclusive scan
+__global__ void __launch_bounds__(256)
+k_wb_children(Cells C, uint32_t* src, uint32_t lf, uint32_t lc, const uint32_t* counts, const uint32_t* members, uint32_t next_first)
+{
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= lc) return;
+    const uint32_t kids = C.info[lf + j] & 15u;
+    const uint32_t child = next_first + counts[j];
+    C.first_child[lf + j] = kids ? child : 0u;
+    for (uint32_t k = 0; k < kids; k++) src[child + k] = members[8 * (size_t)j + k];
+}
+
+// bottom-up: records below each node (its block, padded to an even count, and the blocks below)
+__global__ void __launch_bounds__(256)
+k_wb_size(Cells C, uint32_t lf, uint32_t lc)
+{
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= lc) return;
+    const uint32_t node = lf + j, kids = C.info[node] & 15u, first = C.first_child[node];
+    uint32_t size = kids ? (kids + 1u) & ~1u : 0u;
+    for (uint32_t k = 0; k < kids; k++) size += C.size[first + k];
+    C.size[node] = size;
+}
+
+__global__ void __launch_bounds__(256)
+k_wb_records(const float4* recs, const uint32_t* src, Cells C, uint32_t n_nodes, float4* wrecs)
+{
+    const uint32_t node = blockIdx.x * blockDim.x + threadIdx.x;
+    if (node >= n_nodes) return;
+    const float4* s = recs + 4 * (size_t)src[node];
+    float4* q = wrecs + 4 * (size_t)C.rec[node];
+    float4 q3 = s[3];
+    const uint32_t kids = C.info[node] & 15u;
+    if (kids) { q3.z = __uint_as_float(C.block[node]); q3.w = __uint_as_float(kids); }
+    q[0] = s[0]; q[1] = s[1]; q[2] = s[2]; q[3] = q3;
+}
+
 // Transform::operator()(Triangle) on the device copy of the caller's vertices (mat.cpp:133-140), renderer.cpp:214-224
 __global__ void __launch_bounds__(256)
 k_ob_transform(float* xyz, size_t n_vertices, M4 t)

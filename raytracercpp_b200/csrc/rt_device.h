@@ -25,7 +25,9 @@ typedef float4 rt_f4;
 typedef rtb::F4 rt_f4;
 #endif
 
-#define RT_STACK_SIZE 160              /* 7 * RT_MAX_TREE_DEPTH + root, rounded up */
+/* 7 * RT_MAX_TREE_DEPTH + root, rounded up.  Also bounds the packet stacks on the wide tree (octree_device.cuh, k_wb_*):
+   a root-to-leaf path there visits a subset of the records of the same path in recs[], so it is never deeper. */
+#define RT_STACK_SIZE 160
 #define RT_LEAF_BIT 0x80000000u
 #ifndef RT_META_TOP                    /* the meta word of an interior record, see scene_layout.h */
 #define RT_META_TOP 0x40000000u

@@ -138,6 +138,7 @@ struct DeviceBuild {
     DevBuf<int32_t> mat;
     DevBuf<unsigned long long> keys[2];
     DevBuf<uint32_t> idx[2], hist, sums, counts, c_begin, c_end, c_first, c_info, c_size, c_rec, c_block;
+    DevBuf<uint32_t> w_src, w_members;        // build_wide_tree: the record of recs[] behind each wide node, a frontier's blocks
     DevBuf<devbuild::Stats> stats;
     bool tris_on_device = false;             // xyz9 / uv6 / mat above hold the caller's current triangles
     std::vector<M4> host_pending;            // transforms applied to the device copy but not yet to RtContext::xyz9
@@ -145,7 +146,7 @@ struct DeviceBuild {
     {
         xyz9.release(); uv6.release(); centroid.release(); c_nr.release(); c_fr.release(); mat.release(); keys[0].release(); keys[1].release();
         idx[0].release(); idx[1].release(); hist.release(); sums.release(); counts.release(); c_begin.release(); c_end.release(); c_first.release();
-        c_info.release(); c_size.release(); c_rec.release(); c_block.release(); stats.release();
+        c_info.release(); c_size.release(); c_rec.release(); c_block.release(); w_src.release(); w_members.release(); stats.release();
     }
 };
 
@@ -165,7 +166,9 @@ struct RtContext {
     bool bvh_valid = false;
     RtBvhInfo info{};
     DevBuf<float4> d_recs, d_tris, d_shade, d_mats, d_top;
-    int top_n = 0;
+    DevBuf<float4> d_wrecs;              // the wide copy of the tree for the packet kernels (build_wide_tree)
+    bool wide_tree = false;              // d_wrecs holds it (RT_OPT_LEAF_SPLIT > 0); else the packets traverse d_recs
+    int top_n = 0;                       // records of the top table, built over the array the packets traverse
     DevBuf<int32_t> d_orig, d_leaf_of;
     std::vector<HostShape> shapes;       // analytic shapes, in the order they were added
     DevBuf<float4> d_shapes;
@@ -322,6 +325,15 @@ SceneView scene_view(const RtContext* ctx)
         sc.tex[i].h = ctx->tex[i].h;
         sc.tex[i].format = ctx->tex[i].format;
     }
+    return sc;
+}
+
+// The view of the packet kernels (packet_trace and the kernels of its work items): the wide tree.  The single-ray kernels
+// keep the reference-shaped recs[], whose traversal tallies are those of the host emulation.
+SceneView packet_view(const RtContext* ctx)
+{
+    SceneView sc = scene_view(ctx);
+    if (ctx->wide_tree) sc.recs = ctx->d_wrecs.p;
     return sc;
 }
 
@@ -554,6 +566,85 @@ cudaError_t grow_keep(DevBuf<T>& b, size_t count, size_t keep, cudaStream_t st)
     return e;
 }
 
+// exclusive scan of `count` counters in place (octree_device.cuh); their sum goes to *total unless it is null
+int scan_counts(RtContext* ctx, uint32_t* data, size_t count, uint32_t* total)
+{
+    using namespace devbuild;
+    DeviceBuild& D = ctx->db;
+    const cudaStream_t st = ctx->stream;
+    const uint32_t blocks = (uint32_t)((count + kScanBlock - 1) / kScanBlock);
+    RT_CUDA(ctx, D.sums.ensure(std::max<uint32_t>(blocks, 1)));
+    k_scan_sums<<<blocks, 1024, 0, st>>>(data, count, D.sums.p);
+    k_scan_top<<<1, 1024, 0, st>>>(D.sums.p, blocks, total);
+    k_scan_apply<<<blocks, 1024, 0, st>>>(data, count, D.sums.p);
+    return RT_OK;
+}
+
+// wrecs[], the wide copy of recs[] that the packet kernels traverse (octree_device.cuh: k_wb_*), and the top table over
+// it.  Runs after either builder has put its n_records records in d_recs; the node arrays of the device build are reused
+// (a wide node is one record of recs[], so n_records bounds their number).
+int build_wide_tree(RtContext* ctx, uint64_t n_records)
+{
+    using namespace devbuild;
+    DeviceBuild& D = ctx->db;
+    const cudaStream_t st = ctx->stream;
+    const size_t cap = (size_t)n_records;
+    RT_CUDA(ctx, D.w_src.ensure(cap)); RT_CUDA(ctx, D.c_first.ensure(cap)); RT_CUDA(ctx, D.c_info.ensure(cap)); RT_CUDA(ctx, D.c_size.ensure(cap));
+    RT_CUDA(ctx, D.c_rec.ensure(cap)); RT_CUDA(ctx, D.c_block.ensure(cap)); RT_CUDA(ctx, D.stats.ensure(1));
+    Cells C;
+    memset(&C, 0, sizeof(C));
+    C.first_child = D.c_first.p; C.info = D.c_info.p; C.size = D.c_size.p; C.rec = D.c_rec.p; C.block = D.c_block.p;
+    {
+        const uint32_t zero = 0u, root_block = 2u;                              // the root node is record 0, its block starts at 2
+        RT_CUDA(ctx, cudaMemcpyAsync(D.w_src.p, &zero, 4, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(C.rec, &zero, 4, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(C.block, &root_block, 4, cudaMemcpyHostToDevice, st));
+        RT_CUDA(ctx, cudaStreamSynchronize(st));                                // the sources are on this stack frame
+    }
+    const float4* recs = ctx->d_recs.p;
+    uint32_t* d_total = (uint32_t*)&D.stats.p->top_n;                           // borrowed until the top table is built
+    std::vector<uint32_t> level_first{0u}, level_count{1u};
+    for (;;) {
+        const uint32_t lf = level_first.back(), lc = level_count.back();
+        RT_CUDA(ctx, D.counts.ensure(lc));
+        RT_CUDA(ctx, D.w_members.ensure(8 * (size_t)lc));
+        k_wb_collapse<<<(lc + 255) / 256, 256, 0, st>>>(recs, D.w_src.p, lf, lc, C.info, D.counts.p, D.w_members.p);
+        if (int r = scan_counts(ctx, D.counts.p, lc, d_total)) return r;
+        uint32_t total = 0;
+        RT_CUDA(ctx, cudaMemcpyAsync(&total, d_total, 4, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaStreamSynchronize(st));
+        if (total == 0) break;
+        if ((size_t)lf + lc + total > cap) return fail(ctx, RT_ERR_STATE, "wide tree: more nodes than child records");
+        k_wb_children<<<(lc + 255) / 256, 256, 0, st>>>(C, D.w_src.p, lf, lc, D.counts.p, D.w_members.p, lf + lc);
+        level_first.push_back(lf + lc); level_count.push_back(total);
+    }
+    const uint32_t n_nodes = level_first.back() + level_count.back();
+    for (int l = (int)level_first.size() - 1; l >= 0; l--)
+        k_wb_size<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, level_first[l], level_count[l]);
+    uint32_t root_size = 0;
+    RT_CUDA(ctx, cudaMemcpyAsync(&root_size, C.size, 4, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    const uint64_t n_wide = 2ull + root_size;
+    RT_CUDA(ctx, ctx->d_wrecs.ensure(4 * n_wide));
+    RT_CUDA(ctx, cudaMemsetAsync(ctx->d_wrecs.p, 0, 4 * n_wide * sizeof(float4), st));
+    Params P;
+    memset(&P, 0, sizeof(P));                                                   // leaf_split 0: k_ob_place skips no level
+    for (size_t l = 0; l < level_first.size(); l++)
+        k_ob_place<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, level_first[l], level_count[l], P);
+    k_wb_records<<<(n_nodes + 255) / 256, 256, 0, st>>>(recs, D.w_src.p, C, n_nodes, (float4*)ctx->d_wrecs.p);
+    k_ob_top_table<<<1, 32, 0, st>>>((float4*)ctx->d_wrecs.p, (float4*)ctx->d_top.p, D.stats.p);
+    uint32_t top_n = 0;
+    RT_CUDA(ctx, cudaMemcpyAsync(&top_n, &D.stats.p->top_n, 4, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(ctx, cudaStreamSynchronize(st));
+    RT_CUDA(ctx, cudaGetLastError());
+    ctx->top_n = (int)top_n;
+    ctx->wide_tree = true;
+    if (getenv("RTB200_TRACE"))
+        fprintf(stderr, "[rtb200] wide tree: %llu records on %zu levels (narrow: %llu)\n", (unsigned long long)n_wide, level_first.size(),
+                (unsigned long long)n_records);
+    return RT_OK;
+}
+
 // rt_build_bvh on the device (octree_device.cuh).  n > 0.
 int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
 {
@@ -602,18 +693,10 @@ int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
     RT_CUDA(ctx, D.hist.ensure(n_hist));
     int cur = 0;
     const int passes = (3 * P.total_depth + 7) / 8;
-    auto scan = [&](uint32_t* data, size_t count, uint32_t* total) -> int {
-        const uint32_t blocks = (uint32_t)((count + kScanBlock - 1) / kScanBlock);
-        RT_CUDA(ctx, D.sums.ensure(std::max<uint32_t>(blocks, 1)));
-        k_scan_sums<<<blocks, 1024, 0, st>>>(data, count, D.sums.p);
-        k_scan_top<<<1, 1024, 0, st>>>(D.sums.p, blocks, total);
-        k_scan_apply<<<blocks, 1024, 0, st>>>(data, count, D.sums.p);
-        return RT_OK;
-    };
     (void)hist_blocks;
     for (int pass = 0; pass < passes; pass++) {
         k_rs_count<<<(n_units + 3) / 4, 128, 0, st>>>(D.keys[cur].p, n32, 8 * pass, n_units, D.hist.p);
-        if (int r = scan(D.hist.p, n_hist, nullptr)) return r;
+        if (int r = scan_counts(ctx, D.hist.p, n_hist, nullptr)) return r;
         k_rs_scatter<<<(n_units + 3) / 4, 128, 0, st>>>(D.keys[cur].p, D.idx[cur].p, n32, 8 * pass, n_units, D.hist.p, D.keys[cur ^ 1].p, D.idx[cur ^ 1].p);
         cur ^= 1;
     }
@@ -657,7 +740,7 @@ int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
         const uint32_t lf = level_first.back(), lc = level_count.back();
         RT_CUDA(ctx, D.counts.ensure(lc));
         k_ob_split<<<(lc + 255) / 256, 256, 0, st>>>(keys, cells_view(), lf, lc, depth, P, D.counts.p, D.stats.p);
-        if (int r = scan(D.counts.p, lc, d_total)) return r;
+        if (int r = scan_counts(ctx, D.counts.p, lc, d_total)) return r;
         uint32_t total = 0;
         RT_CUDA(ctx, cudaMemcpyAsync(&total, d_total, 4, cudaMemcpyDeviceToHost, st));
         RT_CUDA(ctx, cudaStreamSynchronize(st));
@@ -692,16 +775,18 @@ int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
     for (size_t l = 0; l < level_first.size(); l++)
         k_ob_place<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, level_first[l], level_count[l], P);
     k_ob_records<<<(n_cells + 255) / 256, 256, 0, st>>>(C, n_cells, P, (float4*)ctx->d_recs.p);
-    k_ob_top_table<<<1, 32, 0, st>>>((float4*)ctx->d_recs.p, (float4*)ctx->d_top.p, D.stats.p);
+    const bool packets_wide = P.leaf_split > 0;                                 // the top table goes over the array the packets traverse
+    if (!packets_wide) k_ob_top_table<<<1, 32, 0, st>>>((float4*)ctx->d_recs.p, (float4*)ctx->d_top.p, D.stats.p);
     Stats hs;
     F4 root_rec[2];
     RT_CUDA(ctx, cudaMemcpyAsync(&hs, D.stats.p, sizeof(hs), cudaMemcpyDeviceToHost, st));
     RT_CUDA(ctx, cudaMemcpyAsync(root_rec, ctx->d_recs.p, sizeof(root_rec), cudaMemcpyDeviceToHost, st));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
     RT_CUDA(ctx, cudaGetLastError());
+    ctx->top_n = (int)hs.top_n;
+    if (packets_wide) if (int r = build_wide_tree(ctx, n_records)) return r;
     const double t2 = now_ms();
 
-    ctx->top_n = (int)hs.top_n;
     ctx->n_tris = n32;
     ctx->root_lo[0] = root_rec[0].x; ctx->root_lo[1] = root_rec[0].z; ctx->root_lo[2] = root_rec[1].x;
     ctx->root_hi[0] = root_rec[0].y; ctx->root_hi[1] = root_rec[0].w; ctx->root_hi[2] = root_rec[1].y;
@@ -800,7 +885,7 @@ void rt_destroy(RtContext* ctx)
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
-    ctx->d_recs.release(); ctx->d_top.release(); ctx->d_tris.release(); ctx->d_shade.release(); ctx->d_mats.release(); ctx->d_orig.release(); ctx->d_leaf_of.release(); ctx->d_shapes.release();
+    ctx->d_recs.release(); ctx->d_wrecs.release(); ctx->d_top.release(); ctx->d_tris.release(); ctx->d_shade.release(); ctx->d_mats.release(); ctx->d_orig.release(); ctx->d_leaf_of.release(); ctx->d_shapes.release();
     for (auto& t : ctx->tex) if (t.d) cudaFree(t.d);
     ctx->d_super.release(); ctx->d_frame.release(); ctx->db.release(); ctx->d_gz.release(); ctx->d_gn.release(); ctx->d_ao.release();
     for (auto& g : ctx->graphs) cudaGraphExecDestroy(g.exec);
@@ -926,6 +1011,7 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
     if (leaf_max_obj_count < 0) return fail(ctx, RT_ERR_INVALID, "leaf_max_obj_count %d", leaf_max_obj_count);
     const size_t n = ctx->xyz9.size() / 9;
     ctx->bvh_valid = false;                              // whatever happens below, the previous tree is gone
+    ctx->wide_tree = false;
     if (ctx->opt_device_build && n > 0) return build_bvh_device(ctx, max_depth, leaf_max_obj_count);
     apply_pending_host_transforms(ctx);
     double t0 = now_ms();
@@ -955,6 +1041,9 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
     }
     RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     double t2 = now_ms();
+    if (n && ctx->opt_leaf_split > 0)                   // replaces the top table over recs[] by one over wrecs[]
+        if (int r = build_wide_tree(ctx, flat.n_records)) return r;
+    const double wide_ms = now_ms() - t2;
     ctx->n_tris = (uint32_t)n;
     {
         const F4 *q0 = &flat.recs[0], *q1 = &flat.recs[1];                       // (near, far) pairs of the three axis slabs
@@ -967,7 +1056,7 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
     bi.max_depth_reached = flat.max_depth_reached; bi.max_leaf_size = flat.max_leaf_size;
     bi.child_records = flat.n_records;
     bi.device_bytes = (flat.recs.size() + flat.tris.size() + flat.shade.size()) * sizeof(F4) + flat.orig.size() * sizeof(int32_t);
-    bi.build_ms = t1 - t0;
+    bi.build_ms = t1 - t0 + wide_ms;
     bi.upload_ms = t2 - t1;
     ctx->bvh_valid = true;
     return RT_OK;
@@ -1137,6 +1226,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
 
     const FrameView fr = frame_view(ctx, s);
     const SceneView sc = scene_view(ctx);
+    const SceneView scp = packet_view(ctx);
     const bool resolve = fr.factor > 1;
     const bool reflect = ctx->any_reflective && s->shading_method == RT_SHADING;
     if (reflect) if (int r = ensure_stack(ctx, s)) return r;
@@ -1316,7 +1406,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     if (graph_ok) {
         auto put = [&](const void* ptr, size_t n) { key.append((const char*)ptr, n); };
         auto put64 = [&](unsigned long long v) { put(&v, sizeof(v)); };
-        put(&sc, sizeof(sc)); put(&fr, sizeof(fr)); put(&wk, sizeof(wk)); put(qv, sizeof(QueueView) * (size_t)n_lanes); put(&tune, sizeof(tune));
+        put(&sc, sizeof(sc)); put(&scp, sizeof(scp)); put(&fr, sizeof(fr)); put(&wk, sizeof(wk)); put(qv, sizeof(QueueView) * (size_t)n_lanes); put(&tune, sizeof(tune));
         put(&light_map, sizeof(light_map));
         if (!bounds.empty()) put(bounds.data(), bounds.size() * sizeof(uint32_t));
         put64((unsigned long long)tile_size); put64((unsigned long long)tile_mod); put64((unsigned long long)tile_rem); put64((unsigned long long)n_lanes);
@@ -1381,28 +1471,28 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
                 QueueView qf = q;
                 qf.tag = next_tag();
                 ScopedTimer t1(ctx, ST_PRIMARY, st, "  k_primary_fused");
-                if (count) k_primary_fused<true><<<grid_pf, kPrimaryThreads, 0, st>>>(sc, fr, wk, qf, cnt, super, tune);
-                else k_primary_fused<false><<<grid_pf, kPrimaryThreads, 0, st>>>(sc, fr, wk, qf, cnt, super, tune);
+                if (count) k_primary_fused<true><<<grid_pf, kPrimaryThreads, 0, st>>>(scp, fr, wk, qf, cnt, super, tune);
+                else k_primary_fused<false><<<grid_pf, kPrimaryThreads, 0, st>>>(scp, fr, wk, qf, cnt, super, tune);
                 launches++;
             } else {
             if (tune.packets) {
                 ScopedTimer t1(ctx, ST_PRIMARY, st, "  k_primary_packet");
-                const bool use_top = ctx->opt_top_table && sc.top_n > 0;
+                const bool use_top = ctx->opt_top_table && scp.top_n > 0;
                 if (count) {
-                    if (use_top) k_primary_packet<true, true><<<grid_pp, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
-                    else k_primary_packet<true, false><<<grid_pp, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
-                } else if (use_top) k_primary_packet<false, true><<<grid_pp, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
-                else k_primary_packet<false, false><<<grid_pp, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
+                    if (use_top) k_primary_packet<true, true><<<grid_pp, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, super, tune);
+                    else k_primary_packet<true, false><<<grid_pp, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, super, tune);
+                } else if (use_top) k_primary_packet<false, true><<<grid_pp, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, super, tune);
+                else k_primary_packet<false, false><<<grid_pp, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, super, tune);
             } else if (count) k_primary<true><<<grid_primary, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
             else k_primary<false><<<grid_primary, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super, tune);
             launches++;
             if (psplit) {
                 for (int pass = 0; pass < tune.item_passes; pass++) {
                     ScopedTimer t1(ctx, ST_PRIMARY, st, "  k_primary_items");
-                    if (count) k_primary_items<true><<<grid_pitems, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, tune, pass);
-                    else k_primary_items<false><<<grid_pitems, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, tune, pass);
+                    if (count) k_primary_items<true><<<grid_pitems, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, tune, pass);
+                    else k_primary_items<false><<<grid_pitems, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, tune, pass);
                 }
-                k_primary_finish<<<grid_pfinish, kPrimaryThreads, 0, st>>>(sc, fr, wk, q, cnt, super);
+                k_primary_finish<<<grid_pfinish, kPrimaryThreads, 0, st>>>(scp, fr, wk, q, cnt, super);
                 launches += tune.item_passes + 1;
             }
             }
@@ -1454,29 +1544,29 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
                 if (++ctx->frame_serial == 0u) ctx->frame_serial = 1u;
                 qf.tag = ctx->frame_serial;
                 ScopedTimer t1(ctx, ST_SHADE, st, "  k_shade_fused");
-                if (count) k_shade_fused<true><<<grid_sf, kQueueThreads, 0, st>>>(sc, fr, wk, qf, cnt, super, tune);
-                else k_shade_fused<false><<<grid_sf, kQueueThreads, 0, st>>>(sc, fr, wk, qf, cnt, super, tune);
+                if (count) k_shade_fused<true><<<grid_sf, kQueueThreads, 0, st>>>(scp, fr, wk, qf, cnt, super, tune);
+                else k_shade_fused<false><<<grid_sf, kQueueThreads, 0, st>>>(scp, fr, wk, qf, cnt, super, tune);
                 launches++;
             } else {
             if (tune.packets) {
                 ScopedTimer t1(ctx, ST_SHADE, st, "  k_shade_packet");
-                const bool use_top = ctx->opt_top_table && sc.top_n > 0;
+                const bool use_top = ctx->opt_top_table && scp.top_n > 0;
                 if (count) {
-                    if (use_top) k_shade_packet<true, true><<<grid_sp, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
-                    else k_shade_packet<true, false><<<grid_sp, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
-                } else if (use_top) k_shade_packet<false, true><<<grid_sp, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
-                else k_shade_packet<false, false><<<grid_sp, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
+                    if (use_top) k_shade_packet<true, true><<<grid_sp, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super, tune);
+                    else k_shade_packet<true, false><<<grid_sp, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super, tune);
+                } else if (use_top) k_shade_packet<false, true><<<grid_sp, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super, tune);
+                else k_shade_packet<false, false><<<grid_sp, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super, tune);
             } else if (count) k_shade<true><<<grid_shade, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
             else k_shade<false><<<grid_shade, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super, tune);
             launches++;
             if (tail) {
                 for (int pass = 0; pass < tune.item_passes; pass++) {
                     ScopedTimer t1(ctx, ST_SHADE, st, "  k_shade_items");
-                    if (count) k_shade_items<true><<<grid_items, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, tune, pass);
-                    else k_shade_items<false><<<grid_items, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, tune, pass);
+                    if (count) k_shade_items<true><<<grid_items, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, tune, pass);
+                    else k_shade_items<false><<<grid_items, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, tune, pass);
                 }
-                if (count) k_shade_finish<true><<<grid_finish, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super);
-                else k_shade_finish<false><<<grid_finish, kQueueThreads, 0, st>>>(sc, fr, wk, qsorted, cnt, super);
+                if (count) k_shade_finish<true><<<grid_finish, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super);
+                else k_shade_finish<false><<<grid_finish, kQueueThreads, 0, st>>>(scp, fr, wk, qsorted, cnt, super);
                 launches += tune.item_passes + 1;
             }
             }
