@@ -238,6 +238,10 @@ enum {
                                  launch.  Results do not depend on it                                                       */
     RT_OPT_RASTER_UNITS = 17, /* hybrid raster path: first size of the list of work units (row bands of the pieces too large for one
                                  thread); a frame that needs more grows the list and repeats its depth pass.  Default 2^18       */
+    RT_OPT_LIGHT_CULL = 21,   /* 1 (default): shadow packets skip the triangles, and the subtrees holding only triangles, that have the
+                                 point light strictly on their front side: back-face culling rejects every crossing of such a triangle
+                                 on the way to the light.  Per-light masks, rebuilt at the first frame after the light, the tree or
+                                 this option changes.  0: masks with every bit set.  Results do not depend on it            */
     RT_OPT_LEAF_SPLIT = 2     /* n > 0 (default 8): when flattening, octree leaves with more than n triangles get a
                                  device-side median-split sub-hierarchy of groups of <= n triangles; 0 = flatten the
                                  reference's cells and leaves exactly as they are.  Applies to the next rt_build_bvh.

@@ -22,7 +22,7 @@ RT_TEX_SKYBOX_RIGHT, RT_TEX_SKYBOX_LEFT, RT_TEX_SKYBOX_TOP, RT_TEX_SKYBOX_BOTTOM
 RT_TEX_DISPLACEMENT = 11
 RT_OPT_COUNT_WORK, RT_OPT_CHUNK_PIXELS, RT_OPT_LEAF_SPLIT, RT_OPT_REFILL_PRIMARY, RT_OPT_REFILL_SHADE, RT_OPT_TRI_BATCH, RT_OPT_PACKETS = 0, 1, 2, 3, 4, 5, 6
 RT_OPT_PACKET_ROUNDS, RT_OPT_SCREEN_CULL, RT_OPT_LANES, RT_OPT_ITEM_ROUNDS, RT_OPT_PRIMARY_ROUNDS, RT_OPT_FUSED_ITEMS, RT_OPT_TOP_TABLE, RT_OPT_SHADOW_SORT, RT_OPT_DEVICE_BUILD, RT_OPT_ITEM_PASSES = 7, 8, 9, 10, 11, 12, 13, 14, 15, 16
-RT_OPT_RASTER_UNITS, RT_OPT_GRAPH, RT_OPT_PACKET_CULL, RT_OPT_FAN_LANES = 17, 18, 19, 20
+RT_OPT_RASTER_UNITS, RT_OPT_GRAPH, RT_OPT_PACKET_CULL, RT_OPT_FAN_LANES, RT_OPT_LIGHT_CULL = 17, 18, 19, 20, 21
 
 
 class RtError(RuntimeError):

@@ -15,7 +15,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "librtb200.so"
 SOURCES = [CSRC / "rtb200.cu", CSRC / "octree_build.cpp", CSRC / "scene_io.cpp"]
-HEADERS = [CSRC / "kernels.cuh", CSRC / "octree_device.cuh", CSRC / "host_common.h", CSRC / "rt_device.h", CSRC / "rt_math.h", CSRC / "scene_layout.h",
+HEADERS = [CSRC / "kernels.cuh", CSRC / "octree_device.cuh", CSRC / "light_cull.cuh", CSRC / "host_common.h", CSRC / "rt_device.h", CSRC / "rt_math.h", CSRC / "scene_layout.h",
            CSRC / "ssao.cuh", CSRC / "ssao_device.h", CSRC / "raster.cuh", CSRC / "raster_device.h",
            PKG.parent / "include" / "rtb200.h"]
 

@@ -492,7 +492,8 @@ RT_DEV void load_top_table(const SceneView& sc, TopTable& T)
 }
 
 // Per-lane inputs: `active`, ray (o, d), t_max (closest: INFINITY; any: light limit).  Outputs: best (closest) or
-// occluded (any).  For ANY: p / dist2 of the reference predicate.  K points to this warp's stack in shared memory, `top`
+// occluded (any).  For ANY: p / dist2 of the reference predicate; subtrees and triangles whose bit in the per-light masks is
+// clear (sc.blk_occ / sc.tri_occ, light_cull.cuh) cannot occlude and are skipped.  K points to this warp's stack in shared memory, `top`
 // to the CTA's copy of the top table (null: none).
 // The traversal starts at the root cell, or (start_meta != 0) at the cell / leaf (start_link, start_meta).
 // Returns false when the packet used up `max_rounds` cell/leaf rounds without finishing (max_rounds 0: no limit); the
@@ -542,6 +543,7 @@ RT_DEV bool packet_trace(const SceneView& sc, PacketStack& K, const float4* top,
         const float tn = active ? slab_entry(q0, q1, q2, q3, sr, t_max) : INFINITY;
         link = f4_bits(q3.z); meta = f4_bits(q3.w);
         if (__ballot_sync(0xffffffffu, tn != INFINITY) == 0u || (meta & ~(RT_LEAF_BIT | RT_META_TOP)) == 0u) return true;
+        if (ANY && (__ldg(sc.blk_occ) & 1u) == 0u) return true;             // nothing in the scene can occlude the light
     }
     int sp = 0;
     for (;;) {
@@ -595,6 +597,7 @@ RT_DEV bool packet_trace(const SceneView& sc, PacketStack& K, const float4* top,
             if (COUNT && lane == 0 && !in_top) tc.rec_fetch += count;
             __syncwarp();
             uint32_t keep = (1u << count) - 1u;
+            if (ANY) keep &= __ldg(sc.blk_occ + (link >> 1));              // children whose subtree may occlude the light
             if (CULL) {
                 // lane 4 * child + plane: the corner of the child's box that lies farthest along the plane's inward normal
                 const uint32_t child = lane >> 2;
@@ -629,10 +632,15 @@ RT_DEV bool packet_trace(const SceneView& sc, PacketStack& K, const float4* top,
             const uint32_t per_round = CULL ? 8u : 10u;
             for (uint32_t first = 0; first < cnt; first += per_round) {
                 const uint32_t m = min(per_round, cnt - first);
+                uint32_t keep = (1u << m) - 1u;
+                if (ANY) {                                   // the triangles that may occlude the light; none: not even staged
+                    const uint32_t at = link + first;
+                    keep &= __funnelshift_r(__ldg(sc.tri_occ + (at >> 5)), __ldg(sc.tri_occ + (at >> 5) + 1), at & 31u);
+                    if (keep == 0u) continue;
+                }
                 if (lane < 3u * m) K.stage[lane] = RT_LDG4(sc.tris + 3 * (size_t)(link + first) + lane);
                 if (COUNT && lane == 0) tc.tri_fetch += m;
                 __syncwarp();
-                uint32_t keep = (1u << m) - 1u;
                 if (CULL) {
                     const uint32_t tri = lane >> 2;
                     const float4 pl = K.plane[lane & 3u];

@@ -69,6 +69,10 @@ struct SceneView {
     uint32_t n_tris;
     const rt_f4* frag_shade; // hybrid raster path only (raster_device.h): shading records of the clipped pieces being shaded, one per
                              // thread; triangle index n_tris + i means record i here (their texture coordinates are the clipped ones)
+    // Any-hit packet traversal only (light_cull.cuh): which triangles and subtrees may occlude the point light.  tri_occ: bit i
+    // = triangle i; blk_occ[link >> 1]: bit k = child record k of the block that starts at record `link`; byte 0, bit 0 = the root.
+    const uint32_t* tri_occ;
+    const uint8_t* blk_occ;
     TexView tex[RT_TEX_COUNT];
 };
 

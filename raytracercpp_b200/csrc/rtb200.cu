@@ -22,6 +22,7 @@
 #include "kernels.cuh"
 #include "scene_layout.h"
 #include "octree_device.cuh"
+#include "light_cull.cuh"
 #include "ssao.cuh"
 #include "raster.cuh"
 #include "host_common.h"
@@ -168,6 +169,8 @@ struct RtContext {
     DevBuf<float4> d_recs, d_tris, d_shade, d_mats, d_top;
     DevBuf<float4> d_wrecs;              // the wide copy of the tree for the packet kernels (build_wide_tree)
     bool wide_tree = false;              // d_wrecs holds it (RT_OPT_LEAF_SPLIT > 0); else the packets traverse d_recs
+    uint64_t n_wrecs = 0;                // records in d_wrecs
+    uint64_t tree_serial = 0;            // bumped by every build of the tree (rt_build_bvh, rt_transform_triangles)
     int top_n = 0;                       // records of the top table, built over the array the packets traverse
     DevBuf<int32_t> d_orig, d_leaf_of;
     std::vector<HostShape> shapes;       // analytic shapes, in the order they were added
@@ -236,6 +239,15 @@ struct RtContext {
     float proj_fov = 45.0f, proj_aspect = 1.0f;
     bool proj_set = false;
     float root_lo[3] = {0, 0, 0}, root_hi[3] = {0, 0, 0};   // the root cell's axis-aligned box (first three slabs)
+
+    // per-light masks of the shadow packets (light_cull.cuh), over the array the packets traverse; rebuilt at the first frame
+    // after their inputs change
+    bool opt_light_cull = true;          // RT_OPT_LIGHT_CULL
+    DevBuf<uint32_t> d_tri_occ, d_blk_occ, d_rec_parent;
+    struct LightMaskInputs { V3 light; float span; uint32_t all_set; uint64_t tree; } mask_in{}, mask_next{};
+    uint32_t mask_words = 0, mask_recs = 0;   // words of tri_occ, records of the traversed array
+    bool mask_valid = false;
+    uint64_t mask_generation = 0;        // part of the frame-graph key
 
     // batch query staging
     DevBuf<float> b_a, b_b, b_t, b_u, b_v;
@@ -334,7 +346,73 @@ SceneView packet_view(const RtContext* ctx)
 {
     SceneView sc = scene_view(ctx);
     if (ctx->wide_tree) sc.recs = ctx->d_wrecs.p;
+    sc.tri_occ = ctx->d_tri_occ.p;
+    sc.blk_occ = (const uint8_t*)ctx->d_blk_occ.p;
     return sc;
+}
+
+// Decides whether the light-cull masks must be rebuilt for the next frame (the light's bits, the tree, the analytic shapes
+// or RT_OPT_LIGHT_CULL changed) and sizes their buffers.  The rebuild itself is enqueued by build_light_masks on the
+// frame's stream before the frame's launches or graph, never inside a captured graph; mask_generation goes into the graph
+// key, so a graph is only replayed over the masks it was captured with.
+int plan_light_masks(RtContext* ctx, bool& rebuild)
+{
+    RtContext::LightMaskInputs in;
+    memset(&in, 0, sizeof(in));                                               // compared bytewise
+    in.light = ctx->light;
+    in.tree = ctx->tree_serial;
+    in.all_set = ctx->opt_light_cull ? 0u : 1u;
+    // span: the longest shadow ray, from a hit point in the root box or on an analytic sphere (light_cull.cuh)
+    double far2 = 0.0;
+    auto corners = [&](const double lo[3], const double hi[3]) {
+        for (int c = 0; c < 8; c++) {
+            const double x = (c & 1 ? hi[0] : lo[0]) - in.light.x, y = (c & 2 ? hi[1] : lo[1]) - in.light.y, z = (c & 4 ? hi[2] : lo[2]) - in.light.z;
+            far2 = std::max(far2, x * x + y * y + z * z);
+        }
+    };
+    const double rlo[3] = {ctx->root_lo[0], ctx->root_lo[1], ctx->root_lo[2]}, rhi[3] = {ctx->root_hi[0], ctx->root_hi[1], ctx->root_hi[2]};
+    corners(rlo, rhi);
+    for (const HostShape& sh : ctx->shapes) {
+        if (sh.bits >> 31) { in.all_set = 1u; continue; }                      // a plane: hit points anywhere
+        const double r = std::sqrt((double)sh.radius2);
+        const double lo[3] = {sh.a[0] - r, sh.a[1] - r, sh.a[2] - r}, hi[3] = {sh.a[0] + r, sh.a[1] + r, sh.a[2] + r};
+        corners(lo, hi);
+    }
+    in.span = (float)(1.01 * std::sqrt(far2) + 1e-3);
+    if (!std::isfinite(in.span)) in.all_set = 1u;
+    rebuild = !ctx->mask_valid || memcmp(&in, &ctx->mask_in, sizeof(in)) != 0;
+    if (!rebuild) return RT_OK;
+    const uint64_t n_recs = ctx->wide_tree ? ctx->n_wrecs : ctx->info.child_records;
+    ctx->mask_words = ctx->n_tris / 32u + 2u;                                   // + 1: a leaf round reads the word after its bits
+    ctx->mask_recs = (uint32_t)n_recs;
+    RT_CUDA(ctx, ctx->d_tri_occ.ensure(ctx->mask_words));
+    RT_CUDA(ctx, ctx->d_blk_occ.ensure(ctx->mask_recs / 8u + 1u));
+    RT_CUDA(ctx, ctx->d_rec_parent.ensure(ctx->mask_recs));
+    ctx->mask_next = in;
+    ctx->mask_generation++;
+    return RT_OK;
+}
+
+int build_light_masks(RtContext* ctx, cudaStream_t st)
+{
+    using namespace lightcull;
+    ScopedTimer tm(ctx, ST_SHADE, st, "light_mask");
+    const RtContext::LightMaskInputs& in = ctx->mask_next;
+    const uint32_t n_words = ctx->mask_words, n_recs = ctx->mask_recs, blk_bytes = (n_recs / 8u + 1u) * 4u;
+    if (in.all_set) {
+        RT_CUDA(ctx, cudaMemsetAsync(ctx->d_tri_occ.p, 0xff, n_words * sizeof(uint32_t), st));
+        RT_CUDA(ctx, cudaMemsetAsync(ctx->d_blk_occ.p, 0xff, blk_bytes, st));
+    } else {
+        const float4* recs = ctx->wide_tree ? ctx->d_wrecs.p : ctx->d_recs.p;
+        RT_CUDA(ctx, cudaMemsetAsync(ctx->d_blk_occ.p, 0, blk_bytes, st));
+        k_lc_tris<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_tris.p, ctx->n_tris, n_words, in.light, in.span, ctx->d_tri_occ.p);
+        k_lc_parents<<<ctx->sm_count * 8, 256, 0, st>>>(recs, n_recs, ctx->d_rec_parent.p);
+        k_lc_leaves<<<ctx->sm_count * 8, 256, 0, st>>>(recs, n_recs, ctx->d_rec_parent.p, ctx->d_tri_occ.p, ctx->d_blk_occ.p);
+    }
+    RT_CUDA(ctx, cudaGetLastError());
+    ctx->mask_in = in;
+    ctx->mask_valid = true;
+    return RT_OK;
 }
 
 int validate_settings(RtContext* ctx, const RtSettings* s)
@@ -625,6 +703,7 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
     RT_CUDA(ctx, cudaMemcpyAsync(&root_size, C.size, 4, cudaMemcpyDeviceToHost, st));
     RT_CUDA(ctx, cudaStreamSynchronize(st));
     const uint64_t n_wide = 2ull + root_size;
+    ctx->n_wrecs = n_wide;
     RT_CUDA(ctx, ctx->d_wrecs.ensure(4 * n_wide));
     RT_CUDA(ctx, cudaMemsetAsync(ctx->d_wrecs.p, 0, 4 * n_wide * sizeof(float4), st));
     Params P;
@@ -958,6 +1037,7 @@ int rt_set_option(RtContext* ctx, int option, int64_t value)
         ctx->opt_lanes = value == 1 ? kLanes : (int)std::max<int64_t>(value, 1);   // 0: one chunk at a time; 1: the default (2); n: n chunks in flight
         return RT_OK;
     case RT_OPT_GRAPH: ctx->opt_graph = value != 0; return RT_OK;
+    case RT_OPT_LIGHT_CULL: ctx->opt_light_cull = value != 0; return RT_OK;
     case RT_OPT_FAN_LANES: ctx->opt_fan_lanes = value != 0; return RT_OK;
     case RT_OPT_PACKET_CULL:
         if (value < 0 || value > 3) return fail(ctx, RT_ERR_INVALID, "packet cull %lld outside [0,3]", (long long)value);
@@ -1012,6 +1092,7 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
     const size_t n = ctx->xyz9.size() / 9;
     ctx->bvh_valid = false;                              // whatever happens below, the previous tree is gone
     ctx->wide_tree = false;
+    ctx->tree_serial++;
     if (ctx->opt_device_build && n > 0) return build_bvh_device(ctx, max_depth, leaf_max_obj_count);
     apply_pending_host_transforms(ctx);
     double t0 = now_ms();
@@ -1224,6 +1305,9 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     if (ssao && tile_mod != 1) return fail(ctx, RT_ERR_UNSUPPORTED, "enable_ssao needs the whole frame on one GPU: its samples read the z-buffer of neighbouring tiles");
     if (ssao && !ctx->proj_set) return fail(ctx, RT_ERR_STATE, "enable_ssao: the projection has not been set (rt_set_projection)");
 
+    bool rebuild_masks = false;                                                // before the views: it may move the mask buffers
+    if (ctx->tune.packets && s->compute_shadows && s->shading_method == RT_SHADING)
+        if (int r = plan_light_masks(ctx, rebuild_masks)) return r;
     const FrameView fr = frame_view(ctx, s);
     const SceneView sc = scene_view(ctx);
     const SceneView scp = packet_view(ctx);
@@ -1415,7 +1499,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
         put64(ctx->opt_top_table); put64((unsigned long long)(uintptr_t)d_argb_out); put64((unsigned long long)(uintptr_t)super);
         put64((unsigned long long)(uintptr_t)ctx->d_counters.p); put64((unsigned long long)(uintptr_t)pd.host_cnt); put64(g_alloc_generation.load());
         put64((unsigned long long)(uintptr_t)main_stream); put64((unsigned long long)split_cap); put64((unsigned long long)item_cap); put64(px_per_tile);
-        put64((unsigned long long)ctx->stack_limit_set); put64(ctx->opt_fan_lanes);
+        put64((unsigned long long)ctx->stack_limit_set); put64(ctx->opt_fan_lanes); put64(ctx->mask_generation);
         if (ssao) { put(&ctx->proj, sizeof(ctx->proj)); put(&ctx->proj_fov, sizeof(float)); put(&ctx->proj_aspect, sizeof(float)); }
         for (size_t i = 0; i < ctx->graphs.size() && !replay; i++)
             if (ctx->graphs[i].key == key) { replay = true; graph_at = i; }
@@ -1429,6 +1513,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     }
     cudaEvent_t ev_begin = next_event(ctx), ev_end = next_event(ctx);
     RT_CUDA(ctx, cudaEventRecord(ev_begin, st));
+    if (rebuild_masks) if (int r = build_light_masks(ctx, st)) return r;
     auto enqueue = [&]() -> int {
     RT_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, sizeof(ChunkCounters) * std::max<uint32_t>(n_chunks, 1), st));
     if (ssao) { k_gbuffer_clear<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_gz.p, ctx->d_gn.p, (size_t)fr.rw * fr.rh); launches++; }
