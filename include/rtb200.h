@@ -218,8 +218,9 @@ enum {
                                  surface already are neighbours from the light (measured: hair scene shadow stage 18.0 ->
                                  6.8 ms with it, 10 M-triangle sphere 7.3 -> 9.6 ms).  Not used with reflection fans.
                                  Results do not depend on it                                                              */
-    RT_OPT_SCREEN_CULL = 8,   /* 1 (default): primary packets outside the screen-space bound of the scene's root box are
-                                 written as misses without tracing.  Results do not depend on it                        */
+    RT_OPT_SCREEN_CULL = 8,   /* 1 (default): primary packets whose 8x4 sample block no ray can take into the boxes of the
+                                 tree's upper levels, and tiles of only such blocks, are written as misses without
+                                 tracing.  Results do not depend on it                                                  */
     RT_OPT_LANES = 9,         /* wavefront chunks in flight at a time, each on its own stream with its own queues, so one
                                  chunk's kernels fill the SMs the others leave idle while their longest packets finish; the
                                  per-stage times of RtRenderStats then overlap.  0: one chunk at a time; 1 (default): 2 chunks;

@@ -123,9 +123,10 @@ struct WorkView {
     int32_t tiles_x;
     int32_t tile_px;                 // tile side in supersampled pixels (tile_size * factor)
     int32_t patches_per_side;        // ceil(tile_px / kPatch)
-    // Supersampled pixels outside [cull_x0, cull_x1] x [cull_y0, cull_y1] cannot hit the scene: the rectangle is the
-    // screen-space bound of the root cell's box (host side, rt_render_device).  The whole frame when no bound exists.
-    int32_t cull_x0, cull_y0, cull_x1, cull_y1;
+    // The scene's screen coverage (host side, screen_coverage): bit bx % 32 of word by * cover_words + bx / 32 is set when the
+    // rays of the 8x4 block (bx, by) of supersampled pixels can hit the scene.  Null when no bound exists: every block can.
+    const uint32_t* cover;
+    int32_t cover_words;
 };
 
 struct QueueView {
@@ -179,6 +180,15 @@ RT_DEV bool slot_pixel(const WorkView& wk, const FrameView& fr, uint32_t slot, i
     px = (int)(tile % (uint32_t)wk.tiles_x) * wk.tile_px + lx;
     py = (int)(tile / (uint32_t)wk.tiles_x) * wk.tile_px + ly;
     return lx < wk.tile_px && ly < wk.tile_px && px < fr.rw && py < fr.rh;
+}
+
+// The 8x4 block of supersampled pixel (px, py) may hold a hit (WorkView::cover).  The 32 lanes of a packet whose block is
+// aligned to the 8x4 grid read one word.
+RT_DEV bool covered(const WorkView& wk, int px, int py)
+{
+    if (wk.cover == nullptr) return true;
+    const uint32_t w = __ldg(wk.cover + ((uint32_t)py >> 2) * (uint32_t)wk.cover_words + ((uint32_t)px >> 8));
+    return ((w >> (((uint32_t)px >> 3) & 31u)) & 1u) != 0u;
 }
 
 // Refill thresholds of the persistent kernels: a warp fetches new rays when at least this many of its lanes are idle
@@ -758,8 +768,8 @@ k_primary_packet(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCoun
             int px = 0, py = 0;
             const bool active = slot < total && slot_pixel(wk, fr, slot, px, py);
             V3 o = v3(0, 0, 0), d = v3(0, 0, 1);
-            // a block that lies outside the screen-space bound of the scene misses without a ray being set up
-            const bool inside = active && px >= wk.cull_x0 && px <= wk.cull_x1 && py >= wk.cull_y0 && py <= wk.cull_y1;
+            // a block that the scene does not cover misses without a ray being set up
+            const bool inside = active && covered(wk, px, py);
             if (__ballot_sync(0xffffffffu, inside) == 0u) {
                 if (slot < total) {
                     q.slot_tri[slot] = -1;
@@ -2079,8 +2089,8 @@ k_primary_fused(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCount
         int px = 0, py = 0;
         const bool active = slot_pixel(wk, fr, slot, px, py);
         V3 o = v3(0, 0, 0), d = v3(0, 0, 1);
-        // a block that lies outside the screen-space bound of the scene misses without a ray being set up
-        const bool inside = active && px >= wk.cull_x0 && px <= wk.cull_x1 && py >= wk.cull_y0 && py <= wk.cull_y1;
+        // a block that the scene does not cover misses without a ray being set up
+        const bool inside = active && covered(wk, px, py);
         bool deferred = false;
         if (__ballot_sync(0xffffffffu, inside) == 0u) {
             q.slot_tri[slot] = -1;

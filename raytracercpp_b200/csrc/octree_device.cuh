@@ -697,6 +697,21 @@ k_wb_records(const float4* recs, const uint32_t* src, Cells C, uint32_t n_nodes,
     q[0] = s[0]; q[1] = s[1]; q[2] = s[2]; q[3] = q3;
 }
 
+// The box set of the screen coverage (rtb200.cu: screen_coverage): the axis box (padded first three slabs) of every wide node
+// in [0, n) that lies on a level at or below `first_kept` or is a leaf; the others get an empty box.  Every triangle lies in
+// a leaf, and every leaf either lies above that level or below a node of it, so the union of the kept boxes holds them all.
+__global__ void __launch_bounds__(256)
+k_wb_boxes(const float4* recs, const uint32_t* src, const uint32_t* info, uint32_t n, uint32_t first_kept, float* boxes)
+{
+    const uint32_t node = blockIdx.x * blockDim.x + threadIdx.x;
+    if (node >= n) return;
+    const float4 q0 = recs[4 * (size_t)src[node]], q1 = recs[4 * (size_t)src[node] + 1];
+    const bool keep = node >= first_kept || (info[node] & 15u) == 0u;
+    float* b = boxes + 6 * (size_t)node;
+    b[0] = keep ? q0.x : INFINITY; b[1] = keep ? q0.z : INFINITY; b[2] = keep ? q1.x : INFINITY;
+    b[3] = keep ? q0.y : -INFINITY; b[4] = keep ? q0.w : -INFINITY; b[5] = keep ? q1.y : -INFINITY;
+}
+
 // Transform::operator()(Triangle) on the device copy of the caller's vertices (mat.cpp:133-140), renderer.cpp:214-224
 __global__ void __launch_bounds__(256)
 k_ob_transform(float* xyz, size_t n_vertices, M4 t)

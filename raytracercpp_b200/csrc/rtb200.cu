@@ -33,6 +33,7 @@ namespace {
 
 constexpr uint64_t kChunkPixels = 1ull << 28;     // supersampled pixels per wavefront chunk (bounds queue memory: 20 B per pixel)
 constexpr int kMaxChunks = 256;
+constexpr uint32_t kCoverBoxes = 4096;           // the screen coverage's box set: the deepest level of the wide tree with at most this many nodes
 
 thread_local std::string g_create_error;
 std::atomic<unsigned long long> g_alloc_generation{0};   // bumped whenever a device buffer moves: invalidates the captured frame graphs
@@ -90,7 +91,7 @@ struct TileList {
     uint32_t* d_split = nullptr;         // traced tiles first, then the others; `count` entries
     std::vector<uint32_t> split_host;
     uint32_t n_traced = 0;
-    int32_t split_rect[4] = {0, 0, -1, -1};
+    uint64_t split_cover = 0;            // cover_generation the split was made with
     int32_t split_tile_px = 0;
     bool split_valid = false;
     float last_hit_fraction = -1.0f;     // hits per traced ray slot of the last frame rendered with this list (-1: none yet)
@@ -140,6 +141,7 @@ struct DeviceBuild {
     DevBuf<unsigned long long> keys[2];
     DevBuf<uint32_t> idx[2], hist, sums, counts, c_begin, c_end, c_first, c_info, c_size, c_rec, c_block;
     DevBuf<uint32_t> w_src, w_members;        // build_wide_tree: the record of recs[] behind each wide node, a frontier's blocks
+    DevBuf<float> w_boxes;                    // build_wide_tree: the box set of the screen coverage (k_wb_boxes)
     DevBuf<devbuild::Stats> stats;
     bool tris_on_device = false;             // xyz9 / uv6 / mat above hold the caller's current triangles
     std::vector<M4> host_pending;            // transforms applied to the device copy but not yet to RtContext::xyz9
@@ -147,7 +149,7 @@ struct DeviceBuild {
     {
         xyz9.release(); uv6.release(); centroid.release(); c_nr.release(); c_fr.release(); mat.release(); keys[0].release(); keys[1].release();
         idx[0].release(); idx[1].release(); hist.release(); sums.release(); counts.release(); c_begin.release(); c_end.release(); c_first.release();
-        c_info.release(); c_size.release(); c_rec.release(); c_block.release(); w_src.release(); w_members.release(); stats.release();
+        c_info.release(); c_size.release(); c_rec.release(); c_block.release(); w_src.release(); w_members.release(); w_boxes.release(); stats.release();
     }
 };
 
@@ -239,6 +241,17 @@ struct RtContext {
     float proj_fov = 45.0f, proj_aspect = 1.0f;
     bool proj_set = false;
     float root_lo[3] = {0, 0, 0}, root_hi[3] = {0, 0, 0};   // the root cell's axis-aligned box (first three slabs)
+    // The screen coverage of the primary packets (screen_coverage): a box set whose union holds every triangle, taken from the
+    // upper levels of the tree at every build, and one bit per 8x4 block of the supersampled frame, set when the block's rays
+    // can reach a box.  Rebuilt at the first frame after its inputs change, like the light masks.
+    std::vector<float> cover_boxes;      // 6 per box: lo xyz, hi xyz (the records' padded axis slabs)
+    struct CoverInputs { M4 proj_inv, cam_to_world; V3 cam_pos; int32_t rw, rh; uint64_t tree; } cover_in{};
+    bool cover_valid = false;
+    bool cover_bound = false;            // false: no bound exists, every block is traced (wk.cover = null)
+    int32_t cover_words = 0;             // 32-bit words per row of blocks
+    std::vector<uint32_t> h_cover;
+    DevBuf<uint32_t> d_cover;
+    uint64_t cover_generation = 0;       // part of the frame-graph key and of the tile split
 
     // per-light masks of the shadow packets (light_cull.cuh), over the array the packets traverse; rebuilt at the first frame
     // after their inputs change
@@ -469,11 +482,7 @@ int grid_for(const RtContext* ctx, const void* kernel, int threads)
     return ctx->sm_count * per_sm;                 // persistent grid: a whole number of CTAs per SM
 }
 
-// Screen-space bound of the scene for the supersampled frame: every primary ray that can hit the root cell's box goes
-// through a pixel of [x0,x1] x [y0,y1].  The eight corners of the box are taken to camera space (inverse of
-// camera_to_world) and through the projection (inverse of proj_inv) in double precision; two pixels of margin cover
-// the float arithmetic of primary_ray.  No bound (whole frame) when a corner is not safely in front of the camera, when
-// the ray origin is not the projection centre (rt_set_camera accepts any position), or when a matrix is singular.
+// Inverse of a 4x4 row-major matrix (Gauss-Jordan with partial pivoting); false when it is singular.
 bool invert4(const double a[16], double out[16])
 {
     double m[4][8];
@@ -496,38 +505,44 @@ bool invert4(const double a[16], double out[16])
     return true;
 }
 
-void screen_cull_rect(const RtContext* ctx, const FrameView& fr, WorkView& wk)
+// Screen coverage of a box set for the supersampled frame rw x rh.  Bit bx % 32 of word by * words_per_row + bx / 32 of `bits`
+// belongs to the 8x4 block (bx, by) -- the footprint of one primary packet -- and is set when a ray that primary_ray generates
+// for a sample of the block can make tri_test accept a triangle inside one of the boxes (6 floats each: lo xyz, hi xyz).
+// Returns false when no bound can be given and every block must be traced: a matrix is singular, the ray origin is not the
+// projection centre, a line of sight does not project back to its own pixel (rt_set_camera accepts any matrices), or the
+// rounding bounds do not hold.  A box that is not safely in front of the camera covers the whole frame.  DESIGN.md §4
+// derives the margin; `margin_scale` multiplies it (1 = the derived margin).  Everything here is double precision.
+bool screen_coverage(const M4& cam_to_world, const M4& proj_inv, V3 cam_pos, int rw, int rh, const float* boxes, size_t n_boxes,
+                     double margin_scale, std::vector<uint32_t>& bits, int32_t& words_per_row)
 {
-    wk.cull_x0 = 0; wk.cull_y0 = 0; wk.cull_x1 = fr.rw - 1; wk.cull_y1 = fr.rh - 1;
-    if (!ctx->opt_screen_cull) return;
-    if (ctx->n_tris == 0 || !(ctx->root_lo[0] <= ctx->root_hi[0])) { wk.cull_x0 = 1; wk.cull_x1 = 0; return; }   // nothing to hit
+    const int bw = (rw + 7) / 8, bh = (rh + 3) / 4;
+    words_per_row = (bw + 31) / 32;
+    bits.assign((size_t)words_per_row * (size_t)bh, 0u);
+    auto set_blocks = [&](int bx0, int by0, int bx1, int by1) {
+        for (int by = by0; by <= by1; by++) {
+            uint32_t* row = bits.data() + (size_t)by * words_per_row;
+            for (int w = bx0 >> 5; w <= bx1 >> 5; w++) {
+                const int lo = std::max(bx0 - 32 * w, 0), hi = std::min(bx1 - 32 * w, 31);
+                row[w] |= (hi == 31 ? 0xffffffffu : ((1u << (hi + 1)) - 1u)) & ~((1u << lo) - 1u);
+            }
+        }
+    };
+    if (n_boxes == 0) return true;                                              // nothing to hit
     double c2w[16], pinv[16], w2c[16], proj[16];
-    for (int i = 0; i < 16; i++) { c2w[i] = (&ctx->cam_to_world.m[0][0])[i]; pinv[i] = (&ctx->proj_inv.m[0][0])[i]; }
-    if (!invert4(c2w, w2c) || !invert4(pinv, proj)) return;
+    for (int i = 0; i < 16; i++) { c2w[i] = (&cam_to_world.m[0][0])[i]; pinv[i] = (&proj_inv.m[0][0])[i]; }
+    if (!invert4(c2w, w2c) || !invert4(pinv, proj)) return false;
     // the ray origin must be the projection centre: camera_to_world * (0,0,0)
     const double w0 = c2w[15];
-    if (!(std::fabs(w0) > 1e-12)) return;
+    if (!(std::fabs(w0) > 1e-12)) return false;
     const double centre[3] = {c2w[3] / w0, c2w[7] / w0, c2w[11] / w0};
-    const double pos[3] = {ctx->cam_pos.x, ctx->cam_pos.y, ctx->cam_pos.z};
-    double scale = 1.0;
+    const double pos[3] = {cam_pos.x, cam_pos.y, cam_pos.z};
+    double scale = 1.0, dc = 0.0;
     for (int k = 0; k < 3; k++) scale = std::max(scale, std::fabs(centre[k]));
-    for (int k = 0; k < 3; k++) if (std::fabs(centre[k] - pos[k]) > 1e-5 * scale) return;
-    double xmin = 1e300, xmax = -1e300, ymin = 1e300, ymax = -1e300;
-    for (int corner = 0; corner < 8; corner++) {
-        const double p[4] = {corner & 1 ? ctx->root_hi[0] : ctx->root_lo[0], corner & 2 ? ctx->root_hi[1] : ctx->root_lo[1],
-                             corner & 4 ? ctx->root_hi[2] : ctx->root_lo[2], 1.0};
-        double v[4], c[4];
-        for (int i = 0; i < 4; i++) v[i] = w2c[4 * i] * p[0] + w2c[4 * i + 1] * p[1] + w2c[4 * i + 2] * p[2] + w2c[4 * i + 3] * p[3];
-        if (!(std::fabs(v[3]) > 1e-12)) return;
-        for (int i = 0; i < 3; i++) v[i] /= v[3];
-        v[3] = 1.0;
-        for (int i = 0; i < 4; i++) c[i] = proj[4 * i] * v[0] + proj[4 * i + 1] * v[1] + proj[4 * i + 2] * v[2] + proj[4 * i + 3] * v[3];
-        // in front of the camera with margin: clip w is the view depth of a perspective projection
-        if (!(c[3] > 1e-3 * (1.0 + std::fabs(v[2])))) return;
-        const double nx = c[0] / c[3], ny = c[1] / c[3];
-        if (!std::isfinite(nx) || !std::isfinite(ny)) return;
-        xmin = std::min(xmin, nx); xmax = std::max(xmax, nx); ymin = std::min(ymin, ny); ymax = std::max(ymax, ny);
+    for (int k = 0; k < 3; k++) {
+        if (!(std::fabs(centre[k] - pos[k]) <= 1e-5 * scale)) return false;
+        dc += (centre[k] - pos[k]) * (centre[k] - pos[k]);
     }
+    dc = std::sqrt(dc);
     // The bound only means something if the rays primary_ray shoots are the projection's own lines of sight: the ray of
     // NDC (x, y) runs from the view-space origin through proj_inv * (x, y, -1), so every point of it must project back to
     // (x, y) with positive clip w.  That holds for the reference's Perspective; rt_set_camera accepts any matrix
@@ -536,20 +551,165 @@ void screen_cull_rect(const RtContext* ctx, const FrameView& fr, WorkView& wk)
         const double nx = k == 4 ? 0.0 : (k & 1 ? 1.0 : -1.0), ny = k == 4 ? 0.0 : (k & 2 ? 1.0 : -1.0);
         double v[4];
         for (int i = 0; i < 4; i++) v[i] = pinv[4 * i] * nx + pinv[4 * i + 1] * ny - pinv[4 * i + 2] + pinv[4 * i + 3];
-        if (!(std::fabs(v[3]) > 1e-12)) return;
+        if (!(std::fabs(v[3]) > 1e-12)) return false;
         for (int i = 0; i < 3; i++) v[i] /= v[3];
         for (const double along : {1.0, 7.5}) {
             const double q[4] = {v[0] * along, v[1] * along, v[2] * along, 1.0};
             double c[4];
             for (int i = 0; i < 4; i++) c[i] = proj[4 * i] * q[0] + proj[4 * i + 1] * q[1] + proj[4 * i + 2] * q[2] + proj[4 * i + 3] * q[3];
-            if (!(c[3] > 0.0) || !(std::fabs(c[0] / c[3] - nx) < 1e-4) || !(std::fabs(c[1] / c[3] - ny) < 1e-4)) return;
+            if (!(c[3] > 0.0) || !(std::fabs(c[0] / c[3] - nx) < 1e-4) || !(std::fabs(c[1] / c[3] - ny) < 1e-4)) return false;
         }
     }
-    const double px0 = (xmin + 1.0) * 0.5 * fr.rw, px1 = (xmax + 1.0) * 0.5 * fr.rw;
-    const double py0 = (ymin + 1.0) * 0.5 * fr.rh, py1 = (ymax + 1.0) * 0.5 * fr.rh;
-    const double lim = 1e9;
-    wk.cull_x0 = (int32_t)std::max(-lim, std::floor(px0) - 2.0); wk.cull_x1 = (int32_t)std::min(lim, std::ceil(px1) + 2.0);
-    wk.cull_y0 = (int32_t)std::max(-lim, std::floor(py0) - 2.0); wk.cull_y1 = (int32_t)std::min(lim, std::ceil(py1) + 2.0);
+    // Rounding of primary_ray's direction (DESIGN.md §4): bounds on the float error of vs = proj_inv (x, y, -1), of
+    // ws = cam_to_world vs and of ws - cam_pos over the whole frame, from the magnitudes of the matrices' terms.  vs and
+    // ws are linear-fractional in (x, y), so their extremes over the frame are at its corners; both denominators must
+    // keep one sign there.
+    const double eps = 0x1p-24;
+    double VS[3] = {0, 0, 0}, WS[3] = {0, 0, 0}, ws_c[4][3], wmin = 1e300, w2min = 1e300, wsign = 0.0, w2sign = 0.0;
+    for (int k = 0; k < 4; k++) {
+        const double h[4] = {k & 1 ? 1.0 : -1.0, k & 2 ? 1.0 : -1.0, -1.0, 1.0};
+        double vh[4], wh[4];
+        for (int i = 0; i < 4; i++) vh[i] = pinv[4 * i] * h[0] + pinv[4 * i + 1] * h[1] + pinv[4 * i + 2] * h[2] + pinv[4 * i + 3] * h[3];
+        if (k == 0) wsign = vh[3] < 0.0 ? -1.0 : 1.0;
+        if (!(vh[3] * wsign > 0.0)) return false;
+        wmin = std::min(wmin, std::fabs(vh[3]));
+        const double vs[4] = {vh[0] / vh[3], vh[1] / vh[3], vh[2] / vh[3], 1.0};
+        for (int i = 0; i < 4; i++) wh[i] = c2w[4 * i] * vs[0] + c2w[4 * i + 1] * vs[1] + c2w[4 * i + 2] * vs[2] + c2w[4 * i + 3];
+        if (k == 0) w2sign = wh[3] < 0.0 ? -1.0 : 1.0;
+        if (!(wh[3] * w2sign > 0.0)) return false;
+        w2min = std::min(w2min, std::fabs(wh[3]));
+        for (int i = 0; i < 3; i++) {
+            ws_c[k][i] = wh[i] / wh[3];
+            VS[i] = std::max(VS[i], std::fabs(vs[i]));
+            WS[i] = std::max(WS[i], std::fabs(ws_c[k][i]));
+        }
+    }
+    double e1[4], ev[3], e2[4], e3n = 0.0;
+    for (int i = 0; i < 4; i++)                          // 4 products and sums, and the rounding of x and y (2 eps each)
+        e1[i] = 6.0 * eps * (std::fabs(pinv[4 * i]) + std::fabs(pinv[4 * i + 1]) + std::fabs(pinv[4 * i + 2]) + std::fabs(pinv[4 * i + 3]));
+    if (!(wmin > 2.0 * e1[3])) return false;
+    for (int i = 0; i < 3; i++) ev[i] = (e1[i] + VS[i] * e1[3]) / (wmin - e1[3]) + 2.0 * eps * VS[i];   // 1 / w, then * (1 / w)
+    for (int i = 0; i < 4; i++) {
+        double s2 = std::fabs(c2w[4 * i + 3]), p2 = 0.0;
+        for (int j = 0; j < 3; j++) { s2 += std::fabs(c2w[4 * i + j]) * VS[j]; p2 += std::fabs(c2w[4 * i + j]) * ev[j]; }
+        e2[i] = 4.0 * eps * s2 + p2;
+    }
+    if (!(w2min > 2.0 * e2[3])) return false;
+    for (int i = 0; i < 3; i++) {
+        const double ew = (e2[i] + WS[i] * e2[3]) / (w2min - e2[3]) + 2.0 * eps * WS[i];
+        const double e3 = ew + eps * (WS[i] + std::fabs(pos[i]));                  // ws - cam_pos
+        e3n += e3 * e3;
+    }
+    e3n = std::sqrt(e3n);
+    // every ws lies in the plane of the frame's corners: its distance from the camera bounds |ws - cam_pos| from below
+    double u[3], v[3], n[3];
+    for (int i = 0; i < 3; i++) { u[i] = ws_c[1][i] - ws_c[0][i]; v[i] = ws_c[2][i] - ws_c[0][i]; }
+    n[0] = u[1] * v[2] - u[2] * v[1]; n[1] = u[2] * v[0] - u[0] * v[2]; n[2] = u[0] * v[1] - u[1] * v[0];
+    const double nn = std::sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
+    const double lmin = std::fabs(n[0] * (ws_c[0][0] - pos[0]) + n[1] * (ws_c[0][1] - pos[1]) + n[2] * (ws_c[0][2] - pos[2])) / nn;
+    if (!(lmin > 4.0 * e3n)) return false;
+    const double e_dir = 2.0 * e3n / lmin + 5.0 * eps;     // |d - D| for the unit exact direction D; normalize adds 5 eps
+    const double kTriRel = 0x1p-14;                          // tri_test's acceptance outside its triangle, relative
+    const double pos_max = std::max(std::fabs(pos[0]), std::max(std::fabs(pos[1]), std::fabs(pos[2])));
+    const double ndc_slack = 1e-9;                           // the double-precision projection below
+    for (size_t b = 0; b < n_boxes; b++) {
+        const float* bx = boxes + 6 * b;
+        bool finite = true, empty = false;
+        double lo[3], hi[3], bmax = 0.0;
+        for (int k = 0; k < 3; k++) {
+            lo[k] = bx[k]; hi[k] = bx[3 + k];
+            finite &= std::isfinite(lo[k]) && std::isfinite(hi[k]);
+            empty |= lo[k] > hi[k];
+            bmax = std::max(bmax, std::max(std::fabs(lo[k]), std::fabs(hi[k])));
+        }
+        if (empty) continue;                                  // holds nothing: k_wb_boxes' (+inf, -inf) for the nodes it leaves out
+        if (!finite) { set_blocks(0, 0, bw - 1, bh - 1); return true; }
+        double sfar = 0.0;
+        for (int c = 0; c < 8; c++) {
+            double d2 = 0.0;
+            for (int k = 0; k < 3; k++) { const double x = ((c >> k) & 1 ? hi[k] : lo[k]) - pos[k]; d2 += x * x; }
+            sfar = std::max(sfar, std::sqrt(d2));
+        }
+        const double e_tri = kTriRel * (pos_max + bmax + sfar);
+        const double reach = (sfar + e_tri) * (1.0 + 5.0 * eps);                // the farthest accepted point, along the ray
+        const double r = margin_scale * (e_tri + reach * e_dir + dc * (2.0 + reach / lmin));
+        double xmin = 1e300, xmax = -1e300, ymin = 1e300, ymax = -1e300;
+        bool whole = false;
+        for (int c = 0; c < 8 && !whole; c++) {
+            const double p[4] = {(c & 1 ? hi[0] + r : lo[0] - r), (c & 2 ? hi[1] + r : lo[1] - r), (c & 4 ? hi[2] + r : lo[2] - r), 1.0};
+            double vv[4], cc[4];
+            for (int i = 0; i < 4; i++) vv[i] = w2c[4 * i] * p[0] + w2c[4 * i + 1] * p[1] + w2c[4 * i + 2] * p[2] + w2c[4 * i + 3] * p[3];
+            if (!(std::fabs(vv[3]) > 1e-12)) { whole = true; break; }
+            for (int i = 0; i < 3; i++) vv[i] /= vv[3];
+            vv[3] = 1.0;
+            for (int i = 0; i < 4; i++) cc[i] = proj[4 * i] * vv[0] + proj[4 * i + 1] * vv[1] + proj[4 * i + 2] * vv[2] + proj[4 * i + 3] * vv[3];
+            // in front of the camera with margin: clip w is the view depth of a perspective projection
+            if (!(cc[3] > 1e-3 * (1.0 + std::fabs(vv[2])))) { whole = true; break; }
+            const double nx = cc[0] / cc[3], ny = cc[1] / cc[3];
+            if (!std::isfinite(nx) || !std::isfinite(ny)) { whole = true; break; }
+            xmin = std::min(xmin, nx); xmax = std::max(xmax, nx); ymin = std::min(ymin, ny); ymax = std::max(ymax, ny);
+        }
+        if (whole) { set_blocks(0, 0, bw - 1, bh - 1); return true; }
+        // samples whose pixel centre (p + 0.5) / n * 2 - 1 lies in [min, max]
+        const double lim = 1e9;
+        const double px0 = std::ceil(std::max(-lim, (xmin - ndc_slack + 1.0) * 0.5 * rw - 0.5)), px1 = std::floor(std::min(lim, (xmax + ndc_slack + 1.0) * 0.5 * rw - 0.5));
+        const double py0 = std::ceil(std::max(-lim, (ymin - ndc_slack + 1.0) * 0.5 * rh - 0.5)), py1 = std::floor(std::min(lim, (ymax + ndc_slack + 1.0) * 0.5 * rh - 0.5));
+        const int x0 = (int)std::max(0.0, px0), x1 = (int)std::min((double)rw - 1, px1);
+        const int y0 = (int)std::max(0.0, py0), y1 = (int)std::min((double)rh - 1, py1);
+        if (x0 > x1 || y0 > y1) continue;
+        set_blocks(x0 >> 3, y0 >> 2, x1 >> 3, y1 >> 2);
+    }
+    return true;
+}
+
+// Any block of supersampled pixels [x0, x1] x [y0, y1] covered
+bool cover_any(const std::vector<uint32_t>& bits, int32_t words_per_row, int x0, int y0, int x1, int y1)
+{
+    const int bx0 = x0 >> 3, bx1 = x1 >> 3;
+    for (int by = y0 >> 2; by <= y1 >> 2; by++) {
+        const uint32_t* row = bits.data() + (size_t)by * words_per_row;
+        for (int w = bx0 >> 5; w <= bx1 >> 5; w++) {
+            const int lo = std::max(bx0 - 32 * w, 0), hi = std::min(bx1 - 32 * w, 31);
+            if (row[w] & (hi == 31 ? 0xffffffffu : ((1u << (hi + 1)) - 1u)) & ~((1u << lo) - 1u)) return true;
+        }
+    }
+    return false;
+}
+
+// Brings the screen coverage up to date for the frame: rebuilt when the camera, the projection, the frame size or the tree
+// changed, and uploaded on the context's stream before the frame's launches or graph (never inside a capture).  The frame
+// before may still read the old bitmap, so the upload waits for it; a camera that does not move costs nothing.
+int update_cover(RtContext* ctx, const FrameView& fr)
+{
+    RtContext::CoverInputs in;
+    memset(&in, 0, sizeof(in));                                               // compared bytewise
+    in.proj_inv = ctx->proj_inv; in.cam_to_world = ctx->cam_to_world; in.cam_pos = ctx->cam_pos;
+    in.rw = fr.rw; in.rh = fr.rh; in.tree = ctx->tree_serial;
+    if (ctx->cover_valid && memcmp(&in, &ctx->cover_in, sizeof(in)) == 0) return RT_OK;
+    ctx->cover_valid = false;
+    const double t0 = now_ms();
+    ctx->cover_bound = screen_coverage(ctx->cam_to_world, ctx->proj_inv, ctx->cam_pos, fr.rw, fr.rh, ctx->cover_boxes.data(),
+                                       ctx->cover_boxes.size() / 6, 1.0, ctx->h_cover, ctx->cover_words);
+    const double t1 = now_ms();
+    double t2 = t1;
+    if (ctx->cover_bound) {
+        RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        t2 = now_ms();
+        RT_CUDA(ctx, ctx->d_cover.ensure(ctx->h_cover.size()));
+        RT_CUDA(ctx, cudaMemcpyAsync(ctx->d_cover.p, ctx->h_cover.data(), ctx->h_cover.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    static const bool trace = getenv("RTB200_TRACE") != nullptr;
+    if (trace) {
+        size_t set = 0;
+        for (uint32_t w : ctx->h_cover) set += (size_t)__builtin_popcount(w);
+        const size_t blocks = (size_t)((fr.rw + 7) / 8) * (size_t)((fr.rh + 3) / 4);
+        fprintf(stderr, "[rtb200] screen coverage: %zu boxes, bound %d, %.4f of the blocks covered, build %.3f ms, upload %.3f ms\n",
+                ctx->cover_boxes.size() / 6, (int)ctx->cover_bound, ctx->cover_bound ? (double)set / (double)blocks : 1.0, t1 - t0, now_ms() - t2);
+    }
+    ctx->cover_in = in;
+    ctx->cover_valid = true;
+    ctx->cover_generation++;
+    return RT_OK;
 }
 
 // The shard's tile list on the device (cached).  tile_rem = -1: the lists of ALL tile_mod shards, each padded with
@@ -658,6 +818,12 @@ int scan_counts(RtContext* ctx, uint32_t* data, size_t count, uint32_t* total)
     return RT_OK;
 }
 
+// The box set of the screen coverage when the packets traverse recs[] itself: the root cell's box
+void root_cover_box(RtContext* ctx)
+{
+    ctx->cover_boxes.assign({ctx->root_lo[0], ctx->root_lo[1], ctx->root_lo[2], ctx->root_hi[0], ctx->root_hi[1], ctx->root_hi[2]});
+}
+
 // wrecs[], the wide copy of recs[] that the packet kernels traverse (octree_device.cuh: k_wb_*), and the top table over
 // it.  Runs after either builder has put its n_records records in d_recs; the node arrays of the device build are reused
 // (a wide node is one record of recs[], so n_records bounds their number).
@@ -697,6 +863,18 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
         level_first.push_back(lf + lc); level_count.push_back(total);
     }
     const uint32_t n_nodes = level_first.back() + level_count.back();
+    {
+        // the box set of the screen coverage: the nodes of the deepest level with at most kCoverBoxes of them, and the leaves
+        // above it (k_wb_boxes); one copy to the host per build
+        size_t lv = 0;
+        while (lv + 1 < level_first.size() && level_count[lv + 1] <= kCoverBoxes) lv++;
+        const uint32_t n_box = level_first[lv] + level_count[lv];
+        RT_CUDA(ctx, D.w_boxes.ensure(6 * (size_t)n_box));
+        k_wb_boxes<<<(n_box + 255) / 256, 256, 0, st>>>(recs, D.w_src.p, C.info, n_box, level_first[lv], D.w_boxes.p);
+        ctx->cover_boxes.resize(6 * (size_t)n_box);
+        RT_CUDA(ctx, cudaMemcpyAsync(ctx->cover_boxes.data(), D.w_boxes.p, 6 * (size_t)n_box * sizeof(float), cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaStreamSynchronize(st));
+    }
     for (int l = (int)level_first.size() - 1; l >= 0; l--)
         k_wb_size<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, level_first[l], level_count[l]);
     uint32_t root_size = 0;
@@ -869,6 +1047,7 @@ int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
     ctx->n_tris = n32;
     ctx->root_lo[0] = root_rec[0].x; ctx->root_lo[1] = root_rec[0].z; ctx->root_lo[2] = root_rec[1].x;
     ctx->root_hi[0] = root_rec[0].y; ctx->root_hi[1] = root_rec[0].w; ctx->root_hi[2] = root_rec[1].y;
+    if (!ctx->wide_tree) root_cover_box(ctx);
     RtBvhInfo& bi = ctx->info;
     bi.triangles = n;
     bi.interior = hs.interior;
@@ -1092,6 +1271,7 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
     const size_t n = ctx->xyz9.size() / 9;
     ctx->bvh_valid = false;                              // whatever happens below, the previous tree is gone
     ctx->wide_tree = false;
+    ctx->cover_boxes.clear();
     ctx->tree_serial++;
     if (ctx->opt_device_build && n > 0) return build_bvh_device(ctx, max_depth, leaf_max_obj_count);
     apply_pending_host_transforms(ctx);
@@ -1131,6 +1311,7 @@ int rt_build_bvh(RtContext* ctx, int max_depth, int leaf_max_obj_count)
         ctx->root_lo[0] = q0->x; ctx->root_lo[1] = q0->z; ctx->root_lo[2] = q1->x;
         ctx->root_hi[0] = q0->y; ctx->root_hi[1] = q0->w; ctx->root_hi[2] = q1->y;
     }
+    if (!ctx->wide_tree && n) root_cover_box(ctx);
     RtBvhInfo& bi = ctx->info;
     bi.triangles = n;
     bi.nodes = flat.nodes; bi.leaves = flat.leaves; bi.empty_leaves = flat.empty_leaves; bi.interior = flat.interior;
@@ -1283,6 +1464,24 @@ int rt_set_light(RtContext* ctx, const float position[3])
     return RT_OK;
 }
 
+// screen_coverage for the camera of rt_set_camera, without a context: a host-only entry point of the library, not part of
+// include/rtb200.h, for tests/test_screen_coverage.py.  Writes the bitmap to bits (room for n_words); returns 1 when it
+// bounds the scene, 0 when no bound exists (every block is traced), RT_ERR_INVALID on bad arguments.
+int rt_screen_coverage(const float proj_inv[16], const float cam_to_world[16], const float position[3], int rw, int rh,
+                       const float* boxes, size_t n_boxes, double margin_scale, uint32_t* bits, size_t n_words)
+{
+    if (!proj_inv || !cam_to_world || !position || rw <= 0 || rh <= 0 || (n_boxes && !boxes) || !bits) return RT_ERR_INVALID;
+    M4 pinv, c2w;
+    memcpy(pinv.m, proj_inv, 64);
+    memcpy(c2w.m, cam_to_world, 64);
+    std::vector<uint32_t> out;
+    int32_t words = 0;
+    const bool bound = screen_coverage(c2w, pinv, v3(position[0], position[1], position[2]), rw, rh, boxes, n_boxes, margin_scale, out, words);
+    if (out.size() > n_words) return RT_ERR_INVALID;
+    std::copy(out.begin(), out.end(), bits);
+    return bound ? 1 : 0;
+}
+
 int rt_tile_count(const RtSettings* s, int tile_size, int tile_mod, int tile_rem)
 {
     if (!s || tile_size <= 0 || tile_mod <= 0 || tile_rem < 0 || tile_rem >= tile_mod) return RT_ERR_INVALID;
@@ -1323,19 +1522,22 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     wk.tiles_x = tiles_x;
     wk.tile_px = tile_size * fr.factor;
     wk.patches_per_side = (wk.tile_px + kPatch - 1) / kPatch;
-    screen_cull_rect(ctx, fr, wk);
-    // Tiles outside the screen-space bound of the scene cannot contain a hit: they get no ray slots, no queue entries and
-    // no traversal, only the miss colour (k_fill_miss).  The wavefront below runs over the other tiles.
+    // Tiles without a block that the scene's screen coverage (screen_coverage) marks cannot contain a hit: they get no ray
+    // slots, no queue entries and no traversal, only the miss colour (k_fill_miss).  The wavefront below runs over the other
+    // tiles, and its packets test their own block's bit.
     const bool has_shapes = !ctx->shapes.empty();                             // planes are unbounded: no screen-space bound
-    if (has_shapes) { wk.cull_x0 = 0; wk.cull_y0 = 0; wk.cull_x1 = fr.rw - 1; wk.cull_y1 = fr.rh - 1; }
-    const bool classify = ctx->opt_screen_cull && ctx->tune.packets && tl->count > 0 && !has_shapes && !raster;
+    const bool cull = ctx->opt_screen_cull && ctx->tune.packets && !has_shapes && !raster;
+    if (cull) if (int r = update_cover(ctx, fr)) return r;
+    wk.cover = (cull && ctx->cover_bound) ? ctx->d_cover.p : nullptr;
+    wk.cover_words = wk.cover ? ctx->cover_words : 0;
+    const bool classify = wk.cover != nullptr && tl->count > 0;
     if (classify) {
-        const int32_t rect[4] = {wk.cull_x0, wk.cull_y0, wk.cull_x1, wk.cull_y1};
-        if (!tl->split_valid || memcmp(rect, tl->split_rect, sizeof(rect)) != 0 || tl->split_tile_px != wk.tile_px) {
+        if (!tl->split_valid || tl->split_cover != ctx->cover_generation || tl->split_tile_px != wk.tile_px) {
             std::vector<uint32_t> in, out;
             for (uint32_t tile : owned) {
                 const int x0 = (int)(tile % (uint32_t)tiles_x) * wk.tile_px, y0 = (int)(tile / (uint32_t)tiles_x) * wk.tile_px;
-                const bool hit = !(x0 + wk.tile_px - 1 < rect[0] || x0 > rect[2] || y0 + wk.tile_px - 1 < rect[1] || y0 > rect[3]);
+                const int x1 = std::min(x0 + wk.tile_px, fr.rw) - 1, y1 = std::min(y0 + wk.tile_px, fr.rh) - 1;
+                const bool hit = cover_any(ctx->h_cover, ctx->cover_words, x0, y0, x1, y1);
                 (hit ? in : out).push_back(tile);
             }
             tl->n_traced = (uint32_t)in.size();
@@ -1344,7 +1546,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
             if (!tl->d_split) RT_CUDA(ctx, cudaMalloc((void**)&tl->d_split, tl->count * sizeof(uint32_t)));
             RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));                  // the previous frame may still read the old split
             RT_CUDA(ctx, cudaMemcpy(tl->d_split, tl->split_host.data(), tl->count * sizeof(uint32_t), cudaMemcpyHostToDevice));
-            memcpy(tl->split_rect, rect, sizeof(rect));
+            tl->split_cover = ctx->cover_generation;
             tl->split_tile_px = wk.tile_px;
             tl->split_valid = true;
         }
@@ -1499,7 +1701,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
         put64(ctx->opt_top_table); put64((unsigned long long)(uintptr_t)d_argb_out); put64((unsigned long long)(uintptr_t)super);
         put64((unsigned long long)(uintptr_t)ctx->d_counters.p); put64((unsigned long long)(uintptr_t)pd.host_cnt); put64(g_alloc_generation.load());
         put64((unsigned long long)(uintptr_t)main_stream); put64((unsigned long long)split_cap); put64((unsigned long long)item_cap); put64(px_per_tile);
-        put64((unsigned long long)ctx->stack_limit_set); put64(ctx->opt_fan_lanes); put64(ctx->mask_generation);
+        put64((unsigned long long)ctx->stack_limit_set); put64(ctx->opt_fan_lanes); put64(ctx->mask_generation); put64(ctx->cover_generation);
         if (ssao) { put(&ctx->proj, sizeof(ctx->proj)); put(&ctx->proj_fov, sizeof(float)); put(&ctx->proj_aspect, sizeof(float)); }
         for (size_t i = 0; i < ctx->graphs.size() && !replay; i++)
             if (ctx->graphs[i].key == key) { replay = true; graph_at = i; }
