@@ -135,9 +135,10 @@ typedef struct RtRenderStats {
     float    reflect_ms;
     float    compact_ms;       /* ordered compaction of the hit records into the ray queues */
     float    resolve_ms;
-    /* Filled only when RT_OPT_COUNT_WORK is on (instrumented kernel instantiations, never the timed ones):
-     * 7-slab volume tests and ray/triangle tests the traversal performed, per ray class -- the V and T of
-     * the bytes-per-ray metric 56*V + 36*T (DESIGN.md).  Reflection = fan rays and their shadow rays. */
+    /* Filled only when RT_OPT_COUNT_WORK is on (instrumented kernel instantiations, never the timed ones) and by
+     * rt_render_work_map, which also splits them per pixel: 7-slab volume tests and ray/triangle tests the traversal
+     * performed, per ray class -- the V and T of the bytes-per-ray metric 56*V + 36*T (DESIGN.md).  Reflection = fan rays
+     * and their shadow rays. */
     uint64_t primary_volume_tests, primary_triangle_tests;
     uint64_t shadow_volume_tests, shadow_triangle_tests;
     uint64_t reflection_volume_tests, reflection_triangle_tests;
@@ -175,7 +176,8 @@ const char* rt_last_error(const RtContext* ctx); /* ctx may be NULL for rt_creat
 
 /* Library knobs (no reference counterpart). */
 enum {
-    RT_OPT_COUNT_WORK = 0,    /* 1: run the instrumented kernels and fill the *_tests counters of RtRenderStats */
+    RT_OPT_COUNT_WORK = 0,    /* 1: run the instrumented kernels and fill the *_tests counters of RtRenderStats (per pixel:
+                                 rt_render_work_map)                                                         */
     RT_OPT_CHUNK_PIXELS = 1,  /* supersampled pixels per wavefront chunk (bounds ray-queue memory)             */
     RT_OPT_REFILL_PRIMARY = 3,/* a warp of k_primary / k_shade fetches new rays once this many of its 32 lanes are idle  */
     RT_OPT_REFILL_SHADE = 4,  /* (default 16)                                                                          */
@@ -339,6 +341,26 @@ int rt_set_light(RtContext* ctx, const float position[3]);
  * utils/mainUtils.cpp:6-21).  argb_out: image_width*image_height ARGB32 words, row 0 = bottom row, exactly
  * the layout of Renderer::get_image() (renderer.cpp:1086).  Host pointer; includes the D2H copy. */
 int rt_render(RtContext* ctx, const RtSettings* settings, uint32_t* argb_out, RtRenderStats* stats);
+
+/* Traversal work of one final-resolution pixel: the tests of every ray of its ssaa_factor^2 samples' ray trees, in the
+ * classes of RtRenderStats -- primary: the samples' primary rays; shadow: the depth-0 shadow rays of their hits (in a
+ * hybrid_rasterization_tracing frame: every test of a fragment's rays, as RtRenderStats counts them); reflection: the
+ * reflection-fan rays of every depth and their shadow rays.  Rays of a packet that was split into work items are credited
+ * with what every item tested for them. */
+typedef struct RtPixelWork {
+    uint64_t primary_volume_tests, primary_triangle_tests;
+    uint64_t shadow_volume_tests, shadow_triangle_tests;
+    uint64_t reflection_volume_tests, reflection_triangle_tests;
+} RtPixelWork;   /* 48 bytes */
+
+/* rt_render with the instrumented kernels, plus the per-pixel split of the work counters: a cost heat map of the frame.
+ * work_out: image_width*image_height entries, row 0 = bottom row (the layout of argb_out); for each field, the sum over all
+ * pixels is the RtRenderStats counter of the same name.  The frame is the one rt_render computes, bit for bit, and `stats`
+ * are what rt_render returns with RT_OPT_COUNT_WORK 1 (the call runs the instrumented kernels whatever that option is
+ * and leaves it as it is).  Every other option applies as usual.  Whole frame, one GPU; never captured or replayed as a
+ * frame graph (the cached graphs stay valid).  The device map (48 B per pixel) is kept by the context like the other
+ * frame buffers.  argb_out and stats may be NULL; work_out may not (RT_ERR_INVALID). */
+int rt_render_work_map(RtContext* ctx, const RtSettings* settings, uint32_t* argb_out, RtPixelWork* work_out, RtRenderStats* stats);
 
 /* Same frame, result left in device memory (`d_argb_out` is a device pointer on the context's device).
  * Tile sharding for the multi-GPU path: the frame is cut into tile_size x tile_size final-resolution

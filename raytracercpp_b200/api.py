@@ -90,6 +90,16 @@ class RtRenderStats(C.Structure):
         return 56 * v + 36 * t
 
 
+class RtPixelWork(C.Structure):
+    """Traversal work of one final-resolution pixel (rt_render_work_map), in the classes of RtRenderStats."""
+    _fields_ = [(n, C.c_uint64) for n in ("primary_volume_tests", "primary_triangle_tests", "shadow_volume_tests", "shadow_triangle_tests",
+                                          "reflection_volume_tests", "reflection_triangle_tests")]
+
+
+# numpy view of an array of RtPixelWork: one uint64 field per C field, same names and order
+PIXEL_WORK_DTYPE = np.dtype([(n, np.uint64) for n, _ in RtPixelWork._fields_])
+
+
 class RtBvhInfo(C.Structure):
     _fields_ = [("triangles", C.c_uint64), ("nodes", C.c_uint64), ("leaves", C.c_uint64), ("empty_leaves", C.c_uint64),
                 ("interior", C.c_uint64), ("max_depth_reached", C.c_uint32), ("max_leaf_size", C.c_uint32),
@@ -135,6 +145,7 @@ ABI = {
     "rt_add_plane": (C.c_int, [C.c_void_p, FP, FP, C.c_int32]),
     "rt_clear_analytic_shapes": (C.c_int, [C.c_void_p]),
     "rt_render": (C.c_int, [C.c_void_p, C.POINTER(RtSettings), UP, C.POINTER(RtRenderStats)]),
+    "rt_render_work_map": (C.c_int, [C.c_void_p, C.POINTER(RtSettings), UP, C.POINTER(RtPixelWork), C.POINTER(RtRenderStats)]),
     "rt_render_device": (C.c_int, [C.c_void_p, C.POINTER(RtSettings), C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(RtRenderStats)]),
     "rt_render_device_begin": (C.c_int, [C.c_void_p, C.POINTER(RtSettings), C.c_void_p, C.c_int, C.c_int, C.c_int]),
     "rt_render_device_end": (C.c_int, [C.c_void_p, C.POINTER(RtRenderStats)]),
@@ -159,8 +170,16 @@ ABI = {
 }
 
 
-def bind(lib: C.CDLL) -> C.CDLL:
+# Symbols that another library with this ABI may lack: the kernel emulation under tests/hostsim and builds of earlier
+# commits (A/B experiments) predate them.  A Context method that needs a missing one raises RtError.  librtb200.so of this
+# tree exports every symbol (load_library binds it with require_all; tests/test_abi.py checks the exports).
+OPTIONAL = {"rt_render_work_map"}
+
+
+def bind(lib: C.CDLL, require_all: bool = False) -> C.CDLL:
     for name, (res, args) in ABI.items():
+        if name in OPTIONAL and not require_all and not hasattr(lib, name):
+            continue
         fn = getattr(lib, name)  # AttributeError if the symbol is missing
         fn.restype = res
         fn.argtypes = args
@@ -180,7 +199,7 @@ def load_library(path=None) -> C.CDLL:
         if not LIB_PATH.exists():
             raise FileNotFoundError(f"{LIB_PATH} is missing: run `python -m raytracercpp_b200.build` (needs nvcc). "
                                     "There is no CPU implementation to fall back to.")
-        _LIB = bind(C.CDLL(str(LIB_PATH)))
+        _LIB = bind(C.CDLL(str(LIB_PATH)), require_all=True)
     return _LIB
 
 
@@ -356,6 +375,21 @@ class Context:
         stats = RtRenderStats()
         self._check(self.lib.rt_render(self.h, C.byref(settings), _p(out, C.c_uint32), C.byref(stats)))
         return out, stats
+
+    def render_work_map(self, settings: RtSettings):
+        """rt_render_work_map: the frame of render() from the instrumented kernels, with its traversal work split per pixel.
+        Returns (argb [H, W] uint32, work, stats): `work` is an [H, W] structured array (PIXEL_WORK_DTYPE) whose six uint64
+        fields carry the names of RtPixelWork; row 0 = bottom row, like argb.  For each field, work[name].sum() equals
+        getattr(stats, name)."""
+        if not hasattr(self.lib, "rt_render_work_map"):
+            raise RtError(RT_ERR_UNSUPPORTED, "this library does not export rt_render_work_map")
+        h, w = settings.image_height, settings.image_width
+        out = np.empty((h, w), np.uint32)
+        work = np.empty((h, w), PIXEL_WORK_DTYPE)
+        stats = RtRenderStats()
+        self._check(self.lib.rt_render_work_map(self.h, C.byref(settings), _p(out, C.c_uint32), work.ctypes.data_as(C.POINTER(RtPixelWork)),
+                                                C.byref(stats)))
+        return out, work, stats
 
     def render_device(self, settings: RtSettings, d_ptr: int, tile_size=64, tile_mod=1, tile_rem=0):
         stats = RtRenderStats()

@@ -80,6 +80,9 @@ struct ChunkCounters {               // one per chunk, zeroed before the frame
     unsigned int rounds_hist[2][16]; // bucket b: packets with 2^b <= rounds < 2^(b+1) (bucket 0 also holds 0 rounds)
     unsigned int max_rounds[2];
     unsigned long long max_packet_ns[2], sum_packet_ns[2];
+    // rt_render_work_map only (null in every other frame, read by the COUNT instantiations only): the per-pixel work map, see
+    // credit_work
+    unsigned long long* work_map;
 };
 
 RT_DEV unsigned long long global_ns()
@@ -115,6 +118,40 @@ RT_DEV void flush_work(TraceCounters& tc, unsigned long long* vol, unsigned long
         if (f) atomicAdd(fetch, f);
     }
 }
+
+// Per-pixel work map (rt_render_work_map; COUNT instantiations only).  ChunkCounters::work_map holds one RtPixelWork per
+// final-resolution pixel: six words, (volume tests, triangle tests) of the classes below in the order of RtRenderStats.
+// Each test is credited to the pixel whose sample issued the ray, with the same class as the warp-aggregated totals above,
+// so the map sums to them.  A packet lane (or a work item's lane) credits what its own ray tested: the tallies of
+// TraceCounters are per lane.
+enum { kWorkPrimary = 0, kWorkShadow = 1, kWorkReflection = 2 };
+
+struct WorkMark {                    // a lane's test tallies when its current ray (or item) started
+    unsigned long long v, t;
+};
+RT_DEV WorkMark work_mark(const TraceCounters& tc) { WorkMark m; m.v = tc.vol_tests; m.t = tc.tri_tests; return m; }
+
+// `pix`: the sample's index py * rw + px in the supersampled frame
+RT_DEV void credit_work(const ChunkCounters* cnt, const FrameView& fr, uint32_t pix, int cls, unsigned long long v, unsigned long long t)
+{
+    if ((v | t) == 0ull) return;
+    unsigned long long* map = cnt->work_map;
+    if (map == nullptr) return;
+    const uint32_t rw = (uint32_t)fr.rw, f = (uint32_t)fr.factor;
+    const size_t x = (pix % rw) / f, y = (pix / rw) / f;
+    unsigned long long* w = map + 6 * (y * (size_t)(rw / f) + x) + 2 * cls;
+    if (v) atomicAdd(w, v);
+    if (t) atomicAdd(w + 1, t);
+}
+
+// credits the tests the lane did since `m`, then moves `m` on
+RT_DEV void credit_since(const ChunkCounters* cnt, const FrameView& fr, uint32_t pix, int cls, const TraceCounters& tc, WorkMark& m)
+{
+    credit_work(cnt, fr, pix, cls, tc.vol_tests - m.v, tc.tri_tests - m.t);
+    m = work_mark(tc);
+}
+
+RT_DEV uint32_t sample_index(const FrameView& fr, int px, int py) { return (uint32_t)py * (uint32_t)fr.rw + (uint32_t)px; }
 
 // Which part of the frame a launch covers: owned tiles [tile_begin, tile_end) of the shard's tile list.
 struct WorkView {
@@ -252,6 +289,7 @@ k_primary(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* c
     const uint32_t pps = (uint32_t)wk.patches_per_side;
     const uint32_t total = (wk.tile_end - wk.tile_begin) * pps * pps * (uint32_t)(kPatch * kPatch);   // ray slots of the chunk
     TraceCounters tc = zero_counters();
+    WorkMark wm = work_mark(tc);                                        // COUNT: where the lane's current ray started
     RayState S;
     RayStack K;
     S.mode = RT_MODE_DONE;
@@ -275,6 +313,7 @@ k_primary(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* c
                 if (slot_pixel(wk, fr, slot, px, py)) {
                     V3 o;
                     primary_ray(fr, px, py, o, dir);
+                    if (COUNT) wm = work_mark(tc);
                     closest_begin<COUNT>(sc, o, dir, S, &tc);
                     alive = true;
                     ++traced;
@@ -292,6 +331,7 @@ k_primary(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* c
         // ---- rays that have ended
         if (alive && S.mode == RT_MODE_DONE) {
             alive = false;
+            if (COUNT) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
             const bool hit = closest_found(S) && S.best.t > 0.1f;          // min_t, renderer.cpp:1039-1040
             if (hit) {
                 q.slot_tri[slot] = S.best.tri; q.slot_t[slot] = S.best.t; q.slot_u[slot] = S.best.u; q.slot_v[slot] = S.best.v;
@@ -786,11 +826,13 @@ k_primary_packet(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCoun
             bool occ, live = active;
             unsigned rounds = 0;
             const unsigned long long t0 = COUNT ? global_ns() : 0ull;
+            WorkMark wm = work_mark(tc);
             if (!((tune.cull & 1) != 0 && packet_set_cull(K, active, o, o + d, 0.0f))) packet_no_cull(K);
             const bool finished = packet_trace<false, COUNT, true>(sc, K, top, live, o, d, INFINITY, o, 0.0f, best, occ, tc, overflow, tune.primary_rounds, rounds,
                                                                    0u, 0u, 0x7fffffff, nullptr, nullptr, make_drain(&cnt->next_patch, total, tune.primary_min));
             __syncwarp();
             if (COUNT && lane == 0) note_packet(cnt, 0, rounds, global_ns() - t0);
+            if (COUNT && active) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
             if (!finished) {
                 // out of rounds: the closest hits so far go to a split record, every unvisited cell becomes a work item
                 const unsigned am = __ballot_sync(0xffffffffu, active);
@@ -806,6 +848,7 @@ k_primary_packet(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCoun
                 live = active;                                                 // no room: trace it here, from the root
                 packet_trace<false, COUNT>(sc, K, top, live, o, d, INFINITY, o, 0.0f, best, occ, tc, overflow, 0, rounds);
                 __syncwarp();
+                if (COUNT && active) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
             }
             if (slot < total) {
                 const bool hit = active && best.tri >= 0 && best.t > 0.1f;        // t > 0 (bvh.h:247) and min_t (renderer.cpp:1039)
@@ -860,6 +903,7 @@ k_primary_items(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCount
         HitRec best;
         bool occ, live = active;
         unsigned rounds = 0;
+        WorkMark wm = work_mark(tc);
         if (!((tune.cull & 1) != 0 && packet_set_cull(K, active, o, o + d, 0.0f))) packet_no_cull(K);
         bool finished = packet_trace<false, COUNT, true>(sc, K, top, live, o, d, t_start, o, 0.0f, best, occ, tc, overflow, budget, rounds, item.y, item.z, orig_start,
                                                          nullptr, nullptr, make_drain(&cnt->p_items_next[pass], n, tune.item_min));
@@ -875,6 +919,7 @@ k_primary_items(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCount
             __syncwarp();
             if (active && best.tri >= 0) atomicMin(mine, closest_key(best.t, sc.orig[best.tri]));
         }
+        if (COUNT && active) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
     }
     if (overflow) atomicOr(&cnt->stack_overflow, 1u);
     if (COUNT) flush_work(tc, &cnt->primary_vol, &cnt->primary_tri, &cnt->primary_fetch);
@@ -1403,6 +1448,7 @@ k_shade(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* cnt
     const uint32_t n = cnt->n_hits;
     TraceCounters tc = zero_counters();
     TraceCounters fan = zero_counters();                      // sums of the per-entry records of k_reflect
+    WorkMark wm = work_mark(tc);                              // COUNT: where the lane's current shadow ray started
     RayState S;
     RayStack K;
     S.mode = RT_MODE_DONE;
@@ -1438,6 +1484,7 @@ k_shade(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* cnt
                     mat = hit.mat;
                     S.occluded = false;
                     S.mode = RT_MODE_DONE;
+                    if (COUNT) wm = work_mark(tc);
                     if (fr.s.compute_shadows) any_begin<COUNT>(sc, p, hit.normal, fr.light, S, &tc);
                     alive = true;                             // ends at once when there is no shadow ray to trace
                 }
@@ -1451,6 +1498,7 @@ k_shade(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* cnt
         for (int it = 0; it < kStepsPerCheck; it++) warp_step<true, COUNT>(sc, S, K, &tc, alive, tune);
         if (alive && S.mode == RT_MODE_DONE) {
             alive = false;
+            if (COUNT) credit_since(cnt, fr, pix, kWorkShadow, tc, wm);
             const MatView m = load_material(sc, mat);
             Col refl = col(0.0f);
             if (m.reflection > 0.0f) {
@@ -1461,6 +1509,7 @@ k_shade(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* cnt
                 if (COUNT) {                                   // fan rays are single rays: one fetch per test
                     fan.vol_tests += q.refl_cnt[3 * (size_t)entry + 1]; fan.tri_tests += q.refl_cnt[3 * (size_t)entry + 2];
                     fan.rec_fetch += q.refl_cnt[3 * (size_t)entry + 1]; fan.tri_fetch += q.refl_cnt[3 * (size_t)entry + 2];
+                    credit_work(cnt, fr, pix, kWorkReflection, q.refl_cnt[3 * (size_t)entry + 1], q.refl_cnt[3 * (size_t)entry + 2]);
                 }
             }
             bool occluded = S.occluded;
@@ -1514,7 +1563,7 @@ RT_DEV ShadeLane shade_prepare(const SceneView& sc, const FrameView& fr, const W
 
 template <bool COUNT>
 RT_DEV void shade_store(const SceneView& sc, const FrameView& fr, const QueueView& q, uint32_t entry, const ShadeLane& L, bool occluded,
-                        TraceCounters& fan, uint32_t* super)
+                        TraceCounters& fan, uint32_t* super, const ChunkCounters* cnt)
 {
     if (!L.rt) { super[L.pix] = quantise_argb(L.direct); return; }
     if (sc.n_shapes > 0 && fr.s.compute_shadows && !occluded) occluded = shapes_occlude(sc, L.p, L.nrm, fr.light);   // renderer.cpp:376-397
@@ -1528,6 +1577,7 @@ RT_DEV void shade_store(const SceneView& sc, const FrameView& fr, const QueueVie
         if (COUNT) {                                   // fan rays are single rays: one fetch per test
                     fan.vol_tests += q.refl_cnt[3 * (size_t)entry + 1]; fan.tri_tests += q.refl_cnt[3 * (size_t)entry + 2];
                     fan.rec_fetch += q.refl_cnt[3 * (size_t)entry + 1]; fan.tri_fetch += q.refl_cnt[3 * (size_t)entry + 2];
+                    credit_work(cnt, fr, L.pix, kWorkReflection, q.refl_cnt[3 * (size_t)entry + 1], q.refl_cnt[3 * (size_t)entry + 2]);
                 }
     }
     super[L.pix] = quantise_argb(shade_compose(fr, m, L.direct, occluded, refl));
@@ -1575,6 +1625,7 @@ k_shade_packet(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounte
         L.rt = false; L.p = v3(0, 0, 0); L.nrm = v3(0, 0, 1);
         if (valid) L = shade_prepare(sc, fr, wk, q, entry, true);
         bool occluded = false, deferred = false;
+        WorkMark wm = work_mark(tc);
         if (fr.s.compute_shadows && fr.s.shading_method == RT_SHADING) {
             bool active = valid && L.rt;
             const V3 so = L.p + 1.0e-4f * L.nrm;                               // Renderer::EPSILON, renderer.h:23
@@ -1607,7 +1658,8 @@ k_shade_packet(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounte
                 }
             }
         }
-        if (valid && !deferred) shade_store<COUNT>(sc, fr, q, entry, L, occluded, fan, super);
+        if (COUNT && valid) credit_since(cnt, fr, L.pix, kWorkShadow, tc, wm);
+        if (valid && !deferred) shade_store<COUNT>(sc, fr, q, entry, L, occluded, fan, super, cnt);
     }
     shade_epilogue<COUNT>(cnt, tc, fan, overflow);
 }
@@ -1653,6 +1705,8 @@ k_shade_items(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounter
         HitRec unused;
         bool occluded = false;
         unsigned rounds = 0;
+        const bool mine = active;                                              // COUNT: this lane's ray is traced by the item
+        WorkMark wm = work_mark(tc);
         if (!((tune.cull & 2) != 0 && packet_set_cull(K, active, fr.light, so, 2.0e-4f))) packet_no_cull(K);
         bool finished = packet_trace<true, COUNT, true>(sc, K, top, active, so, sd, t_lim, L.p, dist2, unused, occluded, tc, overflow, budget, rounds,
                                                         item.y, item.z, 0x7fffffff, nullptr, nullptr, make_drain(&cnt->items_next[pass], n, tune.item_min));
@@ -1663,6 +1717,7 @@ k_shade_items(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounter
             occluded = occluded || before;
             __syncwarp();
         }
+        if (COUNT && mine) credit_since(cnt, fr, L.pix, kWorkShadow, tc, wm);
         const unsigned om = __ballot_sync(0xffffffffu, occluded);
         if (om != 0u && lane == 0) atomicOr(&q.split_occ[sidx], om);
     }
@@ -1686,7 +1741,7 @@ k_shade_finish(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounte
         const uint32_t entry = q.split_base[sidx] + lane;
         if (entry < n_hits && ((q.split_active[sidx] >> lane) & 1u) != 0u) {
             const ShadeLane L = shade_prepare(sc, fr, wk, q, entry);
-            shade_store<COUNT>(sc, fr, q, entry, L, ((q.split_occ[sidx] >> lane) & 1u) != 0u, fan, super);
+            shade_store<COUNT>(sc, fr, q, entry, L, ((q.split_occ[sidx] >> lane) & 1u) != 0u, fan, super, cnt);
         }
     }
     shade_epilogue<COUNT>(cnt, tc, fan, 0u);
@@ -1829,6 +1884,8 @@ RT_DEV void shade_item_fused(const SceneView& sc, const FrameView& fr, const Wor
         bool occluded = false;
         unsigned rounds = 0;
         const int budget = item.w + 1u < kFusedGenerations ? item_budget : 0;
+        const bool mine = active;                                              // COUNT: this lane's ray is traced by the item
+        WorkMark wm = work_mark(tc);
         const bool finished = packet_trace<true, COUNT>(sc, K, top, active, so, sd, t_lim, L.p, dist2, unused, occluded, tc, overflow, budget, rounds, item.y, item.z,
                                                         0x7fffffff, &q.split_occ[sidx]);
         __syncwarp();
@@ -1839,6 +1896,7 @@ RT_DEV void shade_item_fused(const SceneView& sc, const FrameView& fr, const Wor
             occluded = occluded || before;
             __syncwarp();
         }
+        if (COUNT && mine) credit_since(cnt, fr, L.pix, kWorkShadow, tc, wm);
         const unsigned om = __ballot_sync(0xffffffffu, occluded);
         if (om != 0u && lane == 0) atomicOr(&q.split_occ[sidx], om);
     }
@@ -1855,7 +1913,7 @@ RT_DEV void shade_item_fused(const SceneView& sc, const FrameView& fr, const Wor
         occ = __shfl_sync(0xffffffffu, occ, 0);
         if (entry < n_hits && ((am >> lane) & 1u) != 0u) {
             const ShadeLane L = shade_prepare(sc, fr, wk, q, entry);
-            shade_store<COUNT>(sc, fr, q, entry, L, ((occ >> lane) & 1u) != 0u, fan, super);
+            shade_store<COUNT>(sc, fr, q, entry, L, ((occ >> lane) & 1u) != 0u, fan, super, cnt);
         }
     }
     if (lane == 0) { __threadfence(); atomicAdd(&cnt->ft[1].done, 1u); }
@@ -1917,6 +1975,7 @@ k_shade_fused(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounter
         L.rt = false; L.p = v3(0, 0, 0); L.nrm = v3(0, 0, 1);
         if (valid) L = shade_prepare(sc, fr, wk, q, entry, true);
         bool occluded = false, deferred = false;
+        WorkMark wm = work_mark(tc);
         if (shadows) {
             bool active = valid && L.rt;
             const V3 so = L.p + 1.0e-4f * L.nrm;                               // Renderer::EPSILON, renderer.h:23
@@ -1947,7 +2006,8 @@ k_shade_fused(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounter
                 }
             }
         }
-        if (valid && !deferred) shade_store<COUNT>(sc, fr, q, entry, L, occluded, fan, super);
+        if (COUNT && valid) credit_since(cnt, fr, L.pix, kWorkShadow, tc, wm);
+        if (valid && !deferred) shade_store<COUNT>(sc, fr, q, entry, L, occluded, fan, super, cnt);
         ++my_packets;
     }
     shade_epilogue<COUNT>(cnt, tc, fan, overflow);
@@ -2010,6 +2070,7 @@ RT_DEV void primary_item_fused(const SceneView& sc, const FrameView& fr, const W
     bool occ, live = active;
     unsigned rounds = 0;
     const int budget = item.w + 1u < kFusedGenerations ? item_budget : 0;
+    WorkMark wm = work_mark(tc);
     const bool finished = packet_trace<false, COUNT>(sc, K, top, live, o, d, t_start, o, 0.0f, best, occ, tc, overflow, budget, rounds, item.y, item.z, orig_start,
                                                      nullptr, q.split_best + (size_t)sidx * 32u);
     __syncwarp();
@@ -2025,6 +2086,7 @@ RT_DEV void primary_item_fused(const SceneView& sc, const FrameView& fr, const W
         __syncwarp();
         if (active && best.tri >= 0) atomicMin(mine, closest_key(best.t, sc.orig[best.tri]));
     }
+    if (COUNT && active) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
     __threadfence();                                                           // this lane's atomicMin before the pending count drops
     __syncwarp();
     uint32_t left = 0;
@@ -2105,6 +2167,7 @@ k_primary_fused(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCount
             bool occ, live = active;
             unsigned rounds = 0;
             const unsigned long long t0 = COUNT ? global_ns() : 0ull;
+            WorkMark wm = work_mark(tc);
             const bool finished = packet_trace<false, COUNT>(sc, K, top, live, o, d, INFINITY, o, 0.0f, best, occ, tc, overflow,
                                                              fq_budget(tune.primary_rounds, rem), rounds);
             __syncwarp();
@@ -2128,6 +2191,7 @@ k_primary_fused(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCount
                     __syncwarp();
                 }
             }
+            if (COUNT && active) credit_since(cnt, fr, sample_index(fr, px, py), kWorkPrimary, tc, wm);
             if (!deferred) {
                 const bool hit = active && best.tri >= 0 && best.t > 0.1f;        // t > 0 (bvh.h:247) and min_t (renderer.cpp:1039)
                 q.slot_tri[slot] = hit ? best.tri : -1;

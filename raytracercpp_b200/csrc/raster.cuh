@@ -138,7 +138,8 @@ k_raster_units(SceneView sc, FrameView fr, RasterView rv, RasterBuffers rb)
 }
 
 // Tallies go to the frame's ChunkCounters (kernels.cuh): traced_primary = fragments whose ray was tested against their piece,
-// n_hits = those that hit it (each casts one shadow ray), refl_* = the fans' rays, shadow_vol / shadow_tri = tests of all of them.
+// n_hits = those that hit it (each casts one shadow ray), refl_* = the fans' rays, shadow_vol / shadow_tri = tests of all of them
+// (and so does the work map of rt_render_work_map: a fragment's tests are all shadow tests of its pixel).
 template <bool COUNT>
 __global__ void __launch_bounds__(128)
 k_raster_shade(SceneView sc, FrameView fr, RasterView rv, RasterBuffers rb, rt_f4* frag_slots, uint32_t* super, float* g_z, V3* g_n,
@@ -159,7 +160,10 @@ k_raster_shade(SceneView sc, FrameView fr, RasterView rv, RasterBuffers rb, rt_f
         super[pix] = quantise_argb(o.colour);
         if (g_z != nullptr) { g_z[pix] = raster_key_depth(key); g_n[pix] = o.normal; }   // renderer.cpp:976-979
         shaded += o.shaded; hits += o.hit; refl += tc.refl_rays; refl_shadow += tc.refl_shadow_rays;
-        if (COUNT) { vol += tc.vol_tests; tri += tc.tri_tests; }
+        if (COUNT) {
+            vol += tc.vol_tests; tri += tc.tri_tests;
+            credit_work(tallies, fr, (uint32_t)pix, kWorkShadow, tc.vol_tests, tc.tri_tests);   // all of a fragment's rays, as the totals
+        }
         overflow |= tc.stack_overflow;
     }
 #pragma unroll

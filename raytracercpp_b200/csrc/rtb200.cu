@@ -262,6 +262,13 @@ struct RtContext {
     bool mask_valid = false;
     uint64_t mask_generation = 0;        // part of the frame-graph key
 
+    // rt_render_work_map: one RtPixelWork per final pixel, allocated at the first call and grown as needed.  Plain cudaMalloc,
+    // not a DevBuf: the map is no input of any captured frame, so (re)allocating it must not invalidate the frame graphs.
+    unsigned long long* d_work_map = nullptr;
+    size_t work_map_pixels = 0;
+    unsigned long long* frame_work_map = nullptr;   // set for the duration of one rt_render_work_map frame: forces COUNT, no graph
+    std::vector<unsigned long long*> work_map_ptrs; // the pointer once per chunk, the source of its copy into the chunks' counters
+
     // batch query staging
     DevBuf<float> b_a, b_b, b_t, b_u, b_v;
     DevBuf<int32_t> b_id;
@@ -1154,6 +1161,7 @@ void rt_destroy(RtContext* ctx)
     if (ctx->lane_fork) cudaEventDestroy(ctx->lane_fork);
     for (auto e : ctx->lane_join) if (e) cudaEventDestroy(e);
     ctx->d_counters.release(); ctx->d_flag.release();
+    if (ctx->d_work_map) cudaFree(ctx->d_work_map);
     ctx->b_a.release(); ctx->b_b.release(); ctx->b_t.release(); ctx->b_u.release(); ctx->b_v.release(); ctx->b_id.release(); ctx->b_occ.release();
     if (ctx->pending.host_cnt) cudaFreeHost(ctx->pending.host_cnt);
     if (ctx->h_frame) cudaFreeHost(ctx->h_frame);
@@ -1670,7 +1678,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     ctx->events_used = 0;
     ctx->timed.clear();
     uint32_t launches = 0;
-    const bool count = ctx->opt_count_work;
+    const bool count = ctx->opt_count_work || ctx->frame_work_map != nullptr;   // a work-map frame runs the instrumented kernels
     Pending& pd = ctx->pending;
     const size_t n_cnt = std::max<uint32_t>(n_chunks, 1);
     if (n_cnt > pd.host_cap) {
@@ -1685,7 +1693,7 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     // and from then on frames with that key are ONE cudaGraphLaunch: a tile shard's 40 short dependent launches otherwise
     // cost more host and launch latency than their kernels run (a 1/8 shard of the 4K frame: 2.2 ms, 0.5 ms of it the chain).
     static const bool trace_env = getenv("RTB200_TRACE") != nullptr;
-    const bool graph_ok = ctx->opt_graph && !raster && !(tune.fused && tune.packets) && !trace_env;
+    const bool graph_ok = ctx->opt_graph && !raster && !(tune.fused && tune.packets) && !trace_env && ctx->frame_work_map == nullptr;
     bool replay = false, capture = false;
     size_t graph_at = 0;
     std::string key;
@@ -1718,6 +1726,11 @@ int rt_render_device_begin(RtContext* ctx, const RtSettings* s, uint32_t* d_argb
     if (rebuild_masks) if (int r = build_light_masks(ctx, st)) return r;
     auto enqueue = [&]() -> int {
     RT_CUDA(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, sizeof(ChunkCounters) * std::max<uint32_t>(n_chunks, 1), st));
+    if (ctx->frame_work_map) {                                                 // every chunk's counters point at the work map
+        ctx->work_map_ptrs.assign(n_cnt, ctx->frame_work_map);
+        RT_CUDA(ctx, cudaMemcpy2DAsync(&ctx->d_counters.p->work_map, sizeof(ChunkCounters), ctx->work_map_ptrs.data(), sizeof(unsigned long long*),
+                                       sizeof(unsigned long long*), n_cnt, cudaMemcpyHostToDevice, st));
+    }
     if (ssao) { k_gbuffer_clear<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_gz.p, ctx->d_gn.p, (size_t)fr.rw * fr.rh); launches++; }
 
     int (&grids)[2][11] = ctx->grids;                                           // per context: its device's occupancy
@@ -2156,6 +2169,36 @@ int rt_render(RtContext* ctx, const RtSettings* s, uint32_t* argb_out, RtRenderS
     if (int r = rt_render_device_begin(ctx, s, ctx->d_frame.p, 64, 1, 0)) return r;
     const int rc = frame_to_host(ctx, ctx->d_frame.p, argb_out, n);           // enqueued behind the kernels; returns when argb_out is complete
     if (int r = rt_render_device_end(ctx, stats)) return r;
+    return rc;
+}
+
+int rt_render_work_map(RtContext* ctx, const RtSettings* s, uint32_t* argb_out, RtPixelWork* work_out, RtRenderStats* stats)
+{
+    if (!ctx) return RT_ERR_INVALID;
+    if (int r = bind(ctx)) return r;
+    if (int r = validate_settings(ctx, s)) return r;
+    if (!work_out) return fail(ctx, RT_ERR_INVALID, "work_out is NULL");
+    const size_t n = (size_t)s->image_width * s->image_height;
+    RT_CUDA(ctx, ctx->d_frame.ensure(n));
+    if (n > ctx->work_map_pixels) {
+        if (ctx->d_work_map) RT_CUDA(ctx, cudaFree(ctx->d_work_map));
+        ctx->d_work_map = nullptr;
+        ctx->work_map_pixels = 0;
+        RT_CUDA(ctx, cudaMalloc((void**)&ctx->d_work_map, n * sizeof(RtPixelWork)));
+        ctx->work_map_pixels = n;
+    }
+    static_assert(sizeof(RtPixelWork) == 6 * sizeof(unsigned long long), "credit_work (kernels.cuh) addresses six words per pixel");
+    RT_CUDA(ctx, cudaMemsetAsync(ctx->d_work_map, 0, n * sizeof(RtPixelWork), ctx->stream));
+    ctx->frame_work_map = ctx->d_work_map;
+    const int rb = rt_render_device_begin(ctx, s, ctx->d_frame.p, 64, 1, 0);
+    ctx->frame_work_map = nullptr;                                              // only this frame: the next one is what it would have been
+    if (rb) return rb;
+    int rc = argb_out ? frame_to_host(ctx, ctx->d_frame.p, argb_out, n) : RT_OK;
+    if (rc == RT_OK) {
+        const cudaError_t e = cudaMemcpyAsync(work_out, ctx->d_work_map, n * sizeof(RtPixelWork), cudaMemcpyDeviceToHost, ctx->stream);
+        if (e != cudaSuccess) rc = fail(ctx, RT_ERR_CUDA, "work map copy: %s", cudaGetErrorString(e));
+    }
+    if (int r = rt_render_device_end(ctx, stats)) return r;                    // waits for the stream: the map copy is complete
     return rc;
 }
 
