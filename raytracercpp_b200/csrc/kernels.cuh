@@ -359,7 +359,7 @@ k_primary(SceneView sc, FrameView fr, WorkView wk, QueueView q, ChunkCounters* c
 struct PacketStack {
     int saved;                      // entries [0, saved) are the unvisited cells of a packet that ran out of rounds
     float4 plane[4];                // the packet's bounding pyramid (packet_set_cull): inside = x * n.x + y * n.y + z * n.z - w >= 0
-    float4 stage[32];               // the cell (<= 8 records) or leaf chunk (<= 10 triangles) being tested, 512 bytes
+    float4 stage[4 * kWideBlock];   // the cell (<= kWideBlock records) or leaf chunk (<= 10 triangles) being tested, 1 KB
     float t[RT_STACK_SIZE];
     uint32_t link[RT_STACK_SIZE];
     uint32_t meta[RT_STACK_SIZE];
@@ -380,7 +380,8 @@ RT_DEV float warp_min(float x)
 // from the apex; every lane's direction in the tangent plane of that axis; the warp's min / max give a rectangle there,
 // its four sides four planes through the apex.  A cell's child whose axis-aligned box (its first three slabs) lies outside
 // one of them cannot be hit by any ray of the packet: packet_trace drops such children with ONE pass in which lane
-// 4 * child + plane tests the box's farthest corner -- all <= 8 children at once, before any per-ray slab arithmetic.
+// 2 * child + pair tests the box's farthest corner against planes 2 * pair and 2 * pair + 1 -- all <= 16 children at once,
+// before any per-ray slab arithmetic.
 // Pure pruning with margins on every rounding (the rectangle is widened, the plane test has a relative and an absolute
 // slack), so results cannot change.  Returns false (warp-uniform) when the packet has no pyramid: no active lane, or a
 // direction more than ~84 degrees off the axis.  `slack`: how far a ray may leave the segment (point -> apex); 0 for primary
@@ -467,7 +468,7 @@ RT_DEV float slab_entry_packet(const float4* rec, const SlabRay& sr, float t_lim
 
 RT_DEV uint32_t ld_vol(const unsigned int* p) { return *((const volatile unsigned int*)p); }
 
-// One cell round of a packet: the (<= 8) staged or top-table records at `rec` are tested by every lane for its own ray; a
+// One cell round of a packet: the (<= kWideBlock) staged or top-table records at `rec` are tested by every lane for its own ray; a
 // child is entered if ANY lane hits it, with the smallest entry distance of the warp as its sort key (one redux.sync);
 // lane 0 keeps the cell's entries [base, sp) of the shared-memory stack sorted by descending distance, so the nearest is
 // popped first.  (Tried instead: the accepted children kept in registers, one per lane, ranked with a shuffle sweep, stored
@@ -633,40 +634,51 @@ RT_DEV bool packet_trace(const SceneView& sc, PacketStack& K, const float4* top,
         }
         if (!(meta & RT_LEAF_BIT)) {
             // ---- one cell.  Its records come from the CTA's top table (the first levels of the tree: no global fetch), or
-            // the warp fetches them with ONE coalesced 128-bit load per lane; either way they are staged in this warp's
-            // shared memory -- swapped into (entry, exit) order when the packet's rays agree on the signs -- and every lane
-            // then tests every child record (broadcast LDS) for its own ray.
+            // the warp fetches them with coalesced 128-bit loads (two per lane for 16 records); either way they are staged in
+            // this warp's shared memory -- swapped into (entry, exit) order when the packet's rays agree on the signs -- and
+            // every lane then tests every child record (broadcast LDS) for its own ray.
             const uint32_t count = meta & RT_META_COUNT_MASK;
             const bool in_top = top != nullptr && (meta & RT_META_TOP) != 0u;
-            if (lane < 4u * count) {
-                float4 v = in_top ? top[4u * ((meta >> RT_META_TOP_SHIFT) & 0xffu) + lane] : RT_LDG4(sc.recs + 4 * (size_t)link + lane);
-                if (swap_lo) { const float t = v.x; v.x = v.y; v.y = t; }
-                if (swap_hi) { const float t = v.z; v.z = v.w; v.w = t; }
-                K.stage[lane] = v;
+            const float4* src = in_top ? top + 4u * ((meta >> RT_META_TOP_SHIFT) & 0xffu) : sc.recs + 4 * (size_t)link;
+#pragma unroll
+            for (uint32_t i = lane; i < 4u * kWideBlock; i += 32u) {
+                if (i < 4u * count) {
+                    float4 v = in_top ? src[i] : RT_LDG4(src + i);
+                    if (swap_lo) { const float t = v.x; v.x = v.y; v.y = t; }
+                    if (swap_hi) { const float t = v.z; v.z = v.w; v.w = t; }
+                    K.stage[i] = v;
+                }
             }
             if (COUNT && lane == 0 && !in_top) tc.rec_fetch += count;
             __syncwarp();
             uint32_t keep = (1u << count) - 1u;
             if (ANY) keep &= __ldg(sc.blk_occ + (link >> 1));              // children whose subtree may occlude the light
             if (CULL) {
-                // lane 4 * child + plane: the corner of the child's box that lies farthest along the plane's inward normal
-                const uint32_t child = lane >> 2;
-                const float4 pl = K.plane[lane & 3u];
+                // lane 2 * child + pair: for planes 2 * pair and 2 * pair + 1, the corner of the child's box that lies farthest
+                // along the plane's inward normal
+                const uint32_t child = lane >> 1;
                 const float4 b0 = K.stage[4u * child];
                 const float2 b1 = *reinterpret_cast<const float2*>(&K.stage[4u * child + 1u]);
                 // (the staged pairs may have been swapped into entry / exit order; slots >= count hold stale records: masked below)
-                const float ax = pl.x * (pl.x > 0.0f ? fmaxf(b0.x, b0.y) : fminf(b0.x, b0.y));
-                const float ay = pl.y * (pl.y > 0.0f ? fmaxf(b0.z, b0.w) : fminf(b0.z, b0.w));
-                const float az = pl.z * (pl.z > 0.0f ? fmaxf(b1.x, b1.y) : fminf(b1.x, b1.y));
-                const bool outside = (ax + ay + az) - pl.w < -4.0e-6f * (fabsf(ax) + fabsf(ay) + fabsf(az) + fabsf(pl.w));
+                const float lx = fminf(b0.x, b0.y), hx = fmaxf(b0.x, b0.y), ly = fminf(b0.z, b0.w), hy = fmaxf(b0.z, b0.w);
+                const float lz = fminf(b1.x, b1.y), hz = fmaxf(b1.x, b1.y);
+                bool outside = false;
+#pragma unroll
+                for (uint32_t h = 0; h < 2u; h++) {
+                    const float4 pl = K.plane[2u * (lane & 1u) + h];
+                    const float ax = pl.x * (pl.x > 0.0f ? hx : lx);
+                    const float ay = pl.y * (pl.y > 0.0f ? hy : ly);
+                    const float az = pl.z * (pl.z > 0.0f ? hz : lz);
+                    outside |= (ax + ay + az) - pl.w < -4.0e-6f * (fabsf(ax) + fabsf(ay) + fabsf(az) + fabsf(pl.w));
+                }
                 unsigned m = __ballot_sync(0xffffffffu, outside);
-                m |= m >> 1;
-                m |= m >> 2;                                 // bit 4k: some plane has child k outside
-                // gather bit 4k of ~m into bit k
-                unsigned in = ~m & 0x11111111u;
-                in = (in | (in >> 3)) & 0x03030303u;
-                in = (in | (in >> 6)) & 0x000f000fu;
-                in = (in | (in >> 12)) & 0xffu;
+                m |= m >> 1;                                 // bit 2k: some plane has child k outside
+                // gather bit 2k of ~m into bit k
+                unsigned in = ~m & 0x55555555u;
+                in = (in | (in >> 1)) & 0x33333333u;
+                in = (in | (in >> 2)) & 0x0f0f0f0fu;
+                in = (in | (in >> 4)) & 0x00ff00ffu;
+                in = (in | (in >> 8)) & 0xffffu;
                 keep &= in;
             }
             const bool fits = ordered ? packet_cell<true, COUNT>(K.stage, count, sr, t_max, active, K, sp, tc, keep)

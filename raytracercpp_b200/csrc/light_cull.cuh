@@ -24,9 +24,10 @@
 //
 // The masks are built over the array the packets traverse (wrecs[], or recs[] with RT_OPT_LEAF_SPLIT 0):
 //   tri_occ[]  one bit per triangle in tris[] order: the triangle may occlude (k_lc_tris);
-//   blk_occ[]  one byte per child block; blocks start at even record indices (k_ob_place, build_wide_tree: the root's block at
-//              2), so byte link >> 1 belongs to the block at `link` alone; bit k = child record k's subtree holds a triangle
-//              that may occlude.  Byte 0 (no block starts at record 0 or 1) holds the root's own bit.
+//   blk_occ[]  one 16-bit entry per child block (blocks hold up to kWideBlock <= 16 records); blocks start at even record
+//              indices (k_ob_place, build_wide_tree: the root's block at 2), so entry link >> 1 belongs to the block at `link`
+//              alone; bit k = child record k's subtree holds a triangle that may occlude.  Entry 0 (no block starts at record 0
+//              or 1) holds the root's own bit.
 // Bottom-up without the builders' level lists: every record learns its parent (k_lc_parents), then every leaf with a
 // triangle that may occlude sets its bit and walks up setting its ancestors' bits (k_lc_leaves); a walk stops at the first bit
 // that was already set, because whoever set it walks on from there.  Each record's bit is set once.
@@ -99,8 +100,8 @@ k_lc_leaves(const float4* recs, uint32_t n_recs, const uint32_t* parent, const u
         uint32_t c = r;
         for (; c != 0u; c = parent[c]) {
             const uint32_t blk = __float_as_uint(recs[4 * (size_t)parent[c] + 3].z);
-            const uint32_t bit = 1u << (8u * ((blk >> 1) & 3u) + (c - blk));
-            if (atomicOr(&blk_words[blk >> 3], bit) & bit) break;
+            const uint32_t bit = 1u << (16u * ((blk >> 1) & 1u) + (c - blk));
+            if (atomicOr(&blk_words[blk >> 2], bit) & bit) break;
         }
         if (c == 0u) atomicOr(&blk_words[0], 1u);
     }

@@ -59,7 +59,7 @@ struct Cells {
     uint32_t* begin;                     // range [begin, end) of the sorted triangle array
     uint32_t* end;
     uint32_t* first_child;               // index of the first child cell (children are consecutive, in octant order)
-    uint32_t* info;                      // nchild | kind << 4 | is_reference_cell << 6
+    uint32_t* info;                      // nchild | kind << 8 | is_reference_cell << 10
     float* nr;                           // 7 per cell
     float* fr;
     uint32_t* size;                      // records below this cell's own record (depth-first span)
@@ -310,7 +310,7 @@ k_ob_refine(Cells C, uint32_t level_first, uint32_t level_count, Params P, const
     const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < level_count; j += warps) {
         const uint32_t cell = level_first + j;
-        if (((C.info[cell] >> 4) & 3u) != kCellDevInterior) continue;
+        if (((C.info[cell] >> 8) & 3u) != kCellDevInterior) continue;
         const uint32_t base = C.begin[cell], n = C.end[cell] - base;
         uint32_t bounds[9];
         int ng = 1;
@@ -366,7 +366,7 @@ k_ob_split(const unsigned long long* keys, Cells C, uint32_t level_first, uint32
     if (j >= level_count) return;
     const uint32_t cell = level_first + j;
     const uint32_t b = C.begin[cell], e = C.end[cell], n = e - b;
-    const bool is_ref = ((C.info[cell] >> 6) & 1u) != 0u;
+    const bool is_ref = ((C.info[cell] >> 10) & 1u) != 0u;
     const bool ref_split = is_ref && n > (uint32_t)P.leaf_max && depth != P.max_depth;              // bvh.h:171-177
     // below the reference's leaves: the host builder's refinement (median cuts into up to 8 groups, k_ob_refine), again and
     // again until a group holds <= leaf_split
@@ -383,7 +383,7 @@ k_ob_split(const unsigned long long* keys, Cells C, uint32_t level_first, uint32
         }
     }
     counts[j] = kids;
-    C.info[cell] = kids | ((ref_split ? kCellRefInterior : dev_split ? kCellDevInterior : kCellLeaf) << 4) | ((is_ref ? 1u : 0u) << 6);
+    C.info[cell] = kids | ((ref_split ? kCellRefInterior : dev_split ? kCellDevInterior : kCellLeaf) << 8) | ((is_ref ? 1u : 0u) << 10);
     if (ref_split) {
         atomicAdd(&st->interior, 1ull);
         atomicAdd(&st->nonempty_children, (unsigned long long)kids);
@@ -402,7 +402,7 @@ k_ob_children(const unsigned long long* keys, Cells C, uint32_t level_first, uin
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= level_count) return;
     const uint32_t cell = level_first + j;
-    const uint32_t kind = (C.info[cell] >> 4) & 3u;
+    const uint32_t kind = (C.info[cell] >> 8) & 3u;
     if (kind == kCellLeaf) { C.first_child[cell] = 0u; return; }
     const uint32_t b = C.begin[cell], e = C.end[cell];
     const int shift = 3 * (P.total_depth - 1 - depth);
@@ -423,7 +423,7 @@ k_ob_children(const unsigned long long* keys, Cells C, uint32_t level_first, uin
         const uint32_t at = o < 8 ? octant_lower_bound(keys, prev, e, shift, o) : e;
         if (at > prev) {
             C.begin[child] = prev; C.end[child] = at;
-            C.info[child] = (kind == kCellRefInterior ? 1u : 0u) << 6;
+            C.info[child] = (kind == kCellRefInterior ? 1u : 0u) << 10;
             child++;
         }
         prev = at;
@@ -439,7 +439,7 @@ k_ob_leaf_order(Cells C, uint32_t n_cells, const uint32_t* idx_in, uint32_t* idx
     const unsigned lane = threadIdx.x & 31u;
     const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t cell = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; cell < n_cells; cell += warps) {
-        if (((C.info[cell] >> 4) & 3u) != kCellLeaf) continue;
+        if (((C.info[cell] >> 8) & 3u) != kCellLeaf) continue;
         const uint32_t b = C.begin[cell], n = C.end[cell] - b;
         for (uint32_t i = lane; i < n; i += 32u) {
             const uint32_t v = idx_in[b + i];
@@ -481,7 +481,7 @@ k_ob_bounds(const float4* tris, Cells C, uint32_t level_first, uint32_t level_co
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= level_count) return;
     const uint32_t cell = level_first + j;
-    const uint32_t info = C.info[cell], kind = (info >> 4) & 3u, kids = info & 15u;
+    const uint32_t info = C.info[cell], kind = (info >> 8) & 3u, kids = info & 0xffu;
     float nr[7], fr[7];
     for (int pl = 0; pl < 7; pl++) { nr[pl] = INFINITY; fr[pl] = -INFINITY; }
     uint32_t size = 0;
@@ -525,7 +525,7 @@ k_ob_place(Cells C, uint32_t level_first, uint32_t level_count, Params P)
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= level_count) return;
     const uint32_t cell = level_first + j;
-    const uint32_t info = C.info[cell], kind = (info >> 4) & 3u, kids = info & 15u;
+    const uint32_t info = C.info[cell], kind = (info >> 8) & 3u, kids = info & 0xffu;
     if (kind == kCellLeaf) return;
     const uint32_t first = C.first_child[cell];
     if (kids == 1u && P.leaf_split > 0) { C.rec[first] = C.rec[cell]; C.block[first] = C.block[cell]; return; }
@@ -557,7 +557,7 @@ k_ob_records(Cells C, uint32_t n_cells, Params P, float4* recs)
 {
     const uint32_t cell = blockIdx.x * blockDim.x + threadIdx.x;
     if (cell >= n_cells) return;
-    const uint32_t info = C.info[cell], kind = (info >> 4) & 3u, kids = info & 15u;
+    const uint32_t info = C.info[cell], kind = (info >> 8) & 3u, kids = info & 0xffu;
     if (kind != kCellLeaf && kids == 1u && P.leaf_split > 0) return;            // skipped level: the child writes this record
     float nr[7], fr[7];
     for (int pl = 0; pl < 7; pl++) {
@@ -600,17 +600,20 @@ __global__ void k_ob_top_table(float4* recs, float4* top, Stats* st)
 }
 
 // ---- wrecs[]: the wide copy of the tree that the packet kernels traverse.  A packet's cell round (pop, fetch, stage,
-// pyramid cull, slab tests, insertion) has a fixed cost sized for 8 children, and a cell of the reference's octree has 2.6
-// on average (10 M-triangle sphere): one round per level.  Every block of wrecs[] is a collapse of the tree below one owner
-// record instead.  Collapse rule: the block starts as the owner's children; repeatedly, the interior member with the
-// largest surface area of its axis box (first three slabs) among those whose children still fit (members - 1 + its count
-// <= 8) is replaced IN PLACE by its children, ties to the lower position; it stops when no member fits.  Members spliced in
-// can be absorbed in turn, so a block may reach several levels down.
+// pyramid cull, slab tests, insertion) has a fixed cost sized for kWideBlock (16) children, and a cell of the reference's
+// octree has 2.6 on average (10 M-triangle sphere): one round per level.  Every block of wrecs[] is a collapse of the tree
+// below one owner record instead.  Collapse rule: the block starts as the owner's children; repeatedly, the interior member
+// with the largest surface area of its axis box (first three slabs) among those whose children still fit (members - 1 + its
+// count <= limit, limit = kWideBlock) is replaced IN PLACE by its children, ties to the lower position; it stops when no
+// member fits.  Members spliced in can be absorbed in turn, so a block may reach several levels down.
 // A node of the wide tree is a record of recs[] (`src`): leaves are copied unchanged (same triangles), interior records
 // get their wide block and member count.  Same pattern as the narrow build: nodes frontier by frontier (k_wb_collapse,
 // scan, k_wb_children), sizes bottom-up (k_wb_size), positions top-down (k_ob_place), then the records (k_wb_records).
-// The nodes on a root-to-leaf path of wrecs[] are a subset of those of the same path in recs[], so the wide tree is never
-// deeper and the packet stack bound of the narrow tree holds.
+// Packet stack: a cell round pops one entry and pushes at most the block's members, so a packet never holds more than
+// 1 + max over root-to-leaf paths of the sum of (members - 1) of the blocks on the path.  Wider blocks can raise that sum
+// above the narrow tree's (a block may absorb a sibling of the path and still advance it by one level), so k_wb_size
+// computes it (`need`) and build_wide_tree lowers the limit until 1 + need fits RT_STACK_SIZE; with limit 1 nothing is
+// absorbed and the bound is the narrow tree's.
 __device__ __forceinline__ bool wb_interior(uint32_t meta) { return !(meta & RT_META_LEAF) && (meta & RT_META_COUNT_MASK) != 0u; }
 
 __device__ __forceinline__ float wb_axis_area(const float4* recs, uint32_t r)      // half the surface area of the axis box
@@ -620,17 +623,17 @@ __device__ __forceinline__ float wb_axis_area(const float4* recs, uint32_t r)   
     return dx * dy + dy * dz + dz * dx;
 }
 
-// members[8 j ..] = the block of node lf + j (a record of recs[] that is interior), counts[j] = its size (0: leaf)
+// members[kWideBlock j ..] = the block of node lf + j (a record of recs[] that is interior), counts[j] = its size (0: leaf)
 __global__ void __launch_bounds__(256)
-k_wb_collapse(const float4* recs, const uint32_t* src, uint32_t lf, uint32_t lc, uint32_t* info, uint32_t* counts, uint32_t* members)
+k_wb_collapse(const float4* recs, const uint32_t* src, uint32_t lf, uint32_t lc, uint32_t limit, uint32_t* info, uint32_t* counts, uint32_t* members)
 {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= lc) return;
     const float4 own = recs[4 * (size_t)src[lf + j] + 3];
     const uint32_t meta = __float_as_uint(own.w);
     if (!wb_interior(meta)) { counts[j] = 0u; info[lf + j] = 0u; return; }
-    uint32_t m[8], kids[8], link[8];
-    float area[8];
+    uint32_t m[kWideBlock], kids[kWideBlock], link[kWideBlock];
+    float area[kWideBlock];
     int n = 0;
     auto put = [&](int at, uint32_t r) {
         const float4 q3 = recs[4 * (size_t)r + 3];
@@ -645,7 +648,7 @@ k_wb_collapse(const float4* recs, const uint32_t* src, uint32_t lf, uint32_t lc,
     for (;;) {
         int best = -1;
         for (int k = 0; k < n; k++)
-            if (kids[k] && n - 1 + (int)kids[k] <= 8 && (best < 0 || area[k] > area[best])) best = k;
+            if (kids[k] && n - 1 + (int)kids[k] <= (int)limit && (best < 0 || area[k] > area[best])) best = k;
         if (best < 0) break;
         const int c = (int)kids[best];
         const uint32_t l = link[best];
@@ -655,9 +658,9 @@ k_wb_collapse(const float4* recs, const uint32_t* src, uint32_t lf, uint32_t lc,
         for (int k = 0; k < c; k++) put(best + k, l + (uint32_t)k);
         n += c - 1;
     }
-    for (int k = 0; k < n; k++) members[8 * (size_t)j + k] = m[k];
+    for (int k = 0; k < n; k++) members[kWideBlock * (size_t)j + k] = m[k];
     counts[j] = (uint32_t)n;
-    info[lf + j] = (uint32_t)n | (kCellRefInterior << 4);
+    info[lf + j] = (uint32_t)n | (kCellRefInterior << 8);
 }
 
 // the members of the frontier's blocks become the next frontier; counts[] now holds the exclusive scan
@@ -666,22 +669,24 @@ k_wb_children(Cells C, uint32_t* src, uint32_t lf, uint32_t lc, const uint32_t* 
 {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= lc) return;
-    const uint32_t kids = C.info[lf + j] & 15u;
+    const uint32_t kids = C.info[lf + j] & 0xffu;
     const uint32_t child = next_first + counts[j];
     C.first_child[lf + j] = kids ? child : 0u;
-    for (uint32_t k = 0; k < kids; k++) src[child + k] = members[8 * (size_t)j + k];
+    for (uint32_t k = 0; k < kids; k++) src[child + k] = members[kWideBlock * (size_t)j + k];
 }
 
-// bottom-up: records below each node (its block, padded to an even count, and the blocks below)
+// bottom-up: records below each node (its block, padded to an even count, and the blocks below) and the stack need of its
+// subtree (max over paths of the sum of members - 1)
 __global__ void __launch_bounds__(256)
-k_wb_size(Cells C, uint32_t lf, uint32_t lc)
+k_wb_size(Cells C, uint32_t* need, uint32_t lf, uint32_t lc)
 {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= lc) return;
-    const uint32_t node = lf + j, kids = C.info[node] & 15u, first = C.first_child[node];
-    uint32_t size = kids ? (kids + 1u) & ~1u : 0u;
-    for (uint32_t k = 0; k < kids; k++) size += C.size[first + k];
+    const uint32_t node = lf + j, kids = C.info[node] & 0xffu, first = C.first_child[node];
+    uint32_t size = kids ? (kids + 1u) & ~1u : 0u, below = 0u;
+    for (uint32_t k = 0; k < kids; k++) { size += C.size[first + k]; below = max(below, need[first + k]); }
     C.size[node] = size;
+    need[node] = kids ? kids - 1u + below : 0u;
 }
 
 __global__ void __launch_bounds__(256)
@@ -692,7 +697,7 @@ k_wb_records(const float4* recs, const uint32_t* src, Cells C, uint32_t n_nodes,
     const float4* s = recs + 4 * (size_t)src[node];
     float4* q = wrecs + 4 * (size_t)C.rec[node];
     float4 q3 = s[3];
-    const uint32_t kids = C.info[node] & 15u;
+    const uint32_t kids = C.info[node] & 0xffu;
     if (kids) { q3.z = __uint_as_float(C.block[node]); q3.w = __uint_as_float(kids); }
     q[0] = s[0]; q[1] = s[1]; q[2] = s[2]; q[3] = q3;
 }
@@ -706,7 +711,7 @@ k_wb_boxes(const float4* recs, const uint32_t* src, const uint32_t* info, uint32
     const uint32_t node = blockIdx.x * blockDim.x + threadIdx.x;
     if (node >= n) return;
     const float4 q0 = recs[4 * (size_t)src[node]], q1 = recs[4 * (size_t)src[node] + 1];
-    const bool keep = node >= first_kept || (info[node] & 15u) == 0u;
+    const bool keep = node >= first_kept || (info[node] & 0xffu) == 0u;
     float* b = boxes + 6 * (size_t)node;
     b[0] = keep ? q0.x : INFINITY; b[1] = keep ? q0.z : INFINITY; b[2] = keep ? q1.x : INFINITY;
     b[3] = keep ? q0.y : -INFINITY; b[4] = keep ? q0.w : -INFINITY; b[5] = keep ? q1.y : -INFINITY;

@@ -25,8 +25,9 @@ typedef float4 rt_f4;
 typedef rtb::F4 rt_f4;
 #endif
 
-/* 7 * RT_MAX_TREE_DEPTH + root, rounded up.  Also bounds the packet stacks on the wide tree (octree_device.cuh, k_wb_*):
-   a root-to-leaf path there visits a subset of the records of the same path in recs[], so it is never deeper. */
+/* 7 * RT_MAX_TREE_DEPTH + root, rounded up.  The packet stacks on the wide tree hold at most 1 + the largest sum of
+   (members - 1) over the blocks of a root-to-leaf path; build_wide_tree computes that bound and keeps it within this size
+   (octree_device.cuh, k_wb_*). */
 #define RT_STACK_SIZE 160
 #define RT_LEAF_BIT 0x80000000u
 #ifndef RT_META_TOP                    /* the meta word of an interior record, see scene_layout.h */
@@ -39,6 +40,11 @@ typedef rtb::F4 rt_f4;
 #endif
 
 namespace rtb {
+
+// Records per block of the wide tree that the packet kernels traverse (octree_device.cuh: k_wb_collapse).  The packet
+// cull gives each child two lanes and the light-cull masks a 16-bit entry per block, so it is at most 16.
+constexpr uint32_t kWideBlock = 16;
+static_assert(kWideBlock >= 8 && kWideBlock <= 16, "wide blocks hold 8..16 records");
 
 #if defined(__CUDACC__)
 RT_DEV uint32_t f4_bits(float f) { return __float_as_uint(f); }
@@ -70,9 +76,9 @@ struct SceneView {
     const rt_f4* frag_shade; // hybrid raster path only (raster_device.h): shading records of the clipped pieces being shaded, one per
                              // thread; triangle index n_tris + i means record i here (their texture coordinates are the clipped ones)
     // Any-hit packet traversal only (light_cull.cuh): which triangles and subtrees may occlude the point light.  tri_occ: bit i
-    // = triangle i; blk_occ[link >> 1]: bit k = child record k of the block that starts at record `link`; byte 0, bit 0 = the root.
+    // = triangle i; blk_occ[link >> 1]: bit k = child record k of the block that starts at record `link`; entry 0, bit 0 = the root.
     const uint32_t* tri_occ;
-    const uint8_t* blk_occ;
+    const uint16_t* blk_occ;
     TexView tex[RT_TEX_COUNT];
 };
 

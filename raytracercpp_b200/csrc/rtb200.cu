@@ -140,7 +140,8 @@ struct DeviceBuild {
     DevBuf<int32_t> mat;
     DevBuf<unsigned long long> keys[2];
     DevBuf<uint32_t> idx[2], hist, sums, counts, c_begin, c_end, c_first, c_info, c_size, c_rec, c_block;
-    DevBuf<uint32_t> w_src, w_members;        // build_wide_tree: the record of recs[] behind each wide node, a frontier's blocks
+    DevBuf<uint32_t> w_src, w_members, w_need; // build_wide_tree: the record of recs[] behind each wide node, a frontier's blocks,
+                                              // each node's packet stack need (k_wb_size)
     DevBuf<float> w_boxes;                    // build_wide_tree: the box set of the screen coverage (k_wb_boxes)
     DevBuf<devbuild::Stats> stats;
     bool tris_on_device = false;             // xyz9 / uv6 / mat above hold the caller's current triangles
@@ -172,6 +173,7 @@ struct RtContext {
     DevBuf<float4> d_wrecs;              // the wide copy of the tree for the packet kernels (build_wide_tree)
     bool wide_tree = false;              // d_wrecs holds it (RT_OPT_LEAF_SPLIT > 0); else the packets traverse d_recs
     uint64_t n_wrecs = 0;                // records in d_wrecs
+    uint32_t wide_stack = 0;             // the most packet stack entries a traversal of d_wrecs can hold (build_wide_tree)
     uint64_t tree_serial = 0;            // bumped by every build of the tree (rt_build_bvh, rt_transform_triangles)
     int top_n = 0;                       // records of the top table, built over the array the packets traverse
     DevBuf<int32_t> d_orig, d_leaf_of;
@@ -367,7 +369,7 @@ SceneView packet_view(const RtContext* ctx)
     SceneView sc = scene_view(ctx);
     if (ctx->wide_tree) sc.recs = ctx->d_wrecs.p;
     sc.tri_occ = ctx->d_tri_occ.p;
-    sc.blk_occ = (const uint8_t*)ctx->d_blk_occ.p;
+    sc.blk_occ = (const uint16_t*)ctx->d_blk_occ.p;
     return sc;
 }
 
@@ -406,7 +408,7 @@ int plan_light_masks(RtContext* ctx, bool& rebuild)
     ctx->mask_words = ctx->n_tris / 32u + 2u;                                   // + 1: a leaf round reads the word after its bits
     ctx->mask_recs = (uint32_t)n_recs;
     RT_CUDA(ctx, ctx->d_tri_occ.ensure(ctx->mask_words));
-    RT_CUDA(ctx, ctx->d_blk_occ.ensure(ctx->mask_recs / 8u + 1u));
+    RT_CUDA(ctx, ctx->d_blk_occ.ensure(ctx->mask_recs / 4u + 1u));             // 16 bits per even record
     RT_CUDA(ctx, ctx->d_rec_parent.ensure(ctx->mask_recs));
     ctx->mask_next = in;
     ctx->mask_generation++;
@@ -418,7 +420,7 @@ int build_light_masks(RtContext* ctx, cudaStream_t st)
     using namespace lightcull;
     ScopedTimer tm(ctx, ST_SHADE, st, "light_mask");
     const RtContext::LightMaskInputs& in = ctx->mask_next;
-    const uint32_t n_words = ctx->mask_words, n_recs = ctx->mask_recs, blk_bytes = (n_recs / 8u + 1u) * 4u;
+    const uint32_t n_words = ctx->mask_words, n_recs = ctx->mask_recs, blk_bytes = (n_recs / 4u + 1u) * 4u;
     if (in.all_set) {
         RT_CUDA(ctx, cudaMemsetAsync(ctx->d_tri_occ.p, 0xff, n_words * sizeof(uint32_t), st));
         RT_CUDA(ctx, cudaMemsetAsync(ctx->d_blk_occ.p, 0xff, blk_bytes, st));
@@ -840,8 +842,8 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
     DeviceBuild& D = ctx->db;
     const cudaStream_t st = ctx->stream;
     const size_t cap = (size_t)n_records;
-    RT_CUDA(ctx, D.w_src.ensure(cap)); RT_CUDA(ctx, D.c_first.ensure(cap)); RT_CUDA(ctx, D.c_info.ensure(cap)); RT_CUDA(ctx, D.c_size.ensure(cap));
-    RT_CUDA(ctx, D.c_rec.ensure(cap)); RT_CUDA(ctx, D.c_block.ensure(cap)); RT_CUDA(ctx, D.stats.ensure(1));
+    RT_CUDA(ctx, D.w_src.ensure(cap)); RT_CUDA(ctx, D.w_need.ensure(cap)); RT_CUDA(ctx, D.c_first.ensure(cap)); RT_CUDA(ctx, D.c_info.ensure(cap));
+    RT_CUDA(ctx, D.c_size.ensure(cap)); RT_CUDA(ctx, D.c_rec.ensure(cap)); RT_CUDA(ctx, D.c_block.ensure(cap)); RT_CUDA(ctx, D.stats.ensure(1));
     Cells C;
     memset(&C, 0, sizeof(C));
     C.first_child = D.c_first.p; C.info = D.c_info.p; C.size = D.c_size.p; C.rec = D.c_rec.p; C.block = D.c_block.p;
@@ -854,20 +856,34 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
     }
     const float4* recs = ctx->d_recs.p;
     uint32_t* d_total = (uint32_t*)&D.stats.p->top_n;                           // borrowed until the top table is built
-    std::vector<uint32_t> level_first{0u}, level_count{1u};
-    for (;;) {
-        const uint32_t lf = level_first.back(), lc = level_count.back();
-        RT_CUDA(ctx, D.counts.ensure(lc));
-        RT_CUDA(ctx, D.w_members.ensure(8 * (size_t)lc));
-        k_wb_collapse<<<(lc + 255) / 256, 256, 0, st>>>(recs, D.w_src.p, lf, lc, C.info, D.counts.p, D.w_members.p);
-        if (int r = scan_counts(ctx, D.counts.p, lc, d_total)) return r;
-        uint32_t total = 0;
-        RT_CUDA(ctx, cudaMemcpyAsync(&total, d_total, 4, cudaMemcpyDeviceToHost, st));
+    std::vector<uint32_t> level_first, level_count;
+    uint32_t root_size = 0, limit = kWideBlock;
+    // the collapse with limit kWideBlock; narrower (limit halved) only when its packet stack bound would exceed RT_STACK_SIZE
+    for (;; limit /= 2u) {
+        level_first.assign(1, 0u); level_count.assign(1, 1u);
+        for (;;) {
+            const uint32_t lf = level_first.back(), lc = level_count.back();
+            RT_CUDA(ctx, D.counts.ensure(lc));
+            RT_CUDA(ctx, D.w_members.ensure(kWideBlock * (size_t)lc));
+            k_wb_collapse<<<(lc + 255) / 256, 256, 0, st>>>(recs, D.w_src.p, lf, lc, limit, C.info, D.counts.p, D.w_members.p);
+            if (int r = scan_counts(ctx, D.counts.p, lc, d_total)) return r;
+            uint32_t total = 0;
+            RT_CUDA(ctx, cudaMemcpyAsync(&total, d_total, 4, cudaMemcpyDeviceToHost, st));
+            RT_CUDA(ctx, cudaStreamSynchronize(st));
+            if (total == 0) break;
+            if ((size_t)lf + lc + total > cap) return fail(ctx, RT_ERR_STATE, "wide tree: more nodes than child records");
+            k_wb_children<<<(lc + 255) / 256, 256, 0, st>>>(C, D.w_src.p, lf, lc, D.counts.p, D.w_members.p, lf + lc);
+            level_first.push_back(lf + lc); level_count.push_back(total);
+        }
+        for (int l = (int)level_first.size() - 1; l >= 0; l--)
+            k_wb_size<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, D.w_need.p, level_first[l], level_count[l]);
+        uint32_t need = 0;
+        RT_CUDA(ctx, cudaMemcpyAsync(&root_size, C.size, 4, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(ctx, cudaMemcpyAsync(&need, D.w_need.p, 4, cudaMemcpyDeviceToHost, st));
         RT_CUDA(ctx, cudaStreamSynchronize(st));
-        if (total == 0) break;
-        if ((size_t)lf + lc + total > cap) return fail(ctx, RT_ERR_STATE, "wide tree: more nodes than child records");
-        k_wb_children<<<(lc + 255) / 256, 256, 0, st>>>(C, D.w_src.p, lf, lc, D.counts.p, D.w_members.p, lf + lc);
-        level_first.push_back(lf + lc); level_count.push_back(total);
+        ctx->wide_stack = need + 1u;
+        if (ctx->wide_stack <= RT_STACK_SIZE) break;
+        if (limit <= 1u) return fail(ctx, RT_ERR_INVALID, "tree too deep for the packet stack (%u > %d entries)", ctx->wide_stack, RT_STACK_SIZE);
     }
     const uint32_t n_nodes = level_first.back() + level_count.back();
     {
@@ -882,11 +898,6 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
         RT_CUDA(ctx, cudaMemcpyAsync(ctx->cover_boxes.data(), D.w_boxes.p, 6 * (size_t)n_box * sizeof(float), cudaMemcpyDeviceToHost, st));
         RT_CUDA(ctx, cudaStreamSynchronize(st));
     }
-    for (int l = (int)level_first.size() - 1; l >= 0; l--)
-        k_wb_size<<<(level_count[l] + 255) / 256, 256, 0, st>>>(C, level_first[l], level_count[l]);
-    uint32_t root_size = 0;
-    RT_CUDA(ctx, cudaMemcpyAsync(&root_size, C.size, 4, cudaMemcpyDeviceToHost, st));
-    RT_CUDA(ctx, cudaStreamSynchronize(st));
     const uint64_t n_wide = 2ull + root_size;
     ctx->n_wrecs = n_wide;
     RT_CUDA(ctx, ctx->d_wrecs.ensure(4 * n_wide));
@@ -904,8 +915,8 @@ int build_wide_tree(RtContext* ctx, uint64_t n_records)
     ctx->top_n = (int)top_n;
     ctx->wide_tree = true;
     if (getenv("RTB200_TRACE"))
-        fprintf(stderr, "[rtb200] wide tree: %llu records on %zu levels (narrow: %llu)\n", (unsigned long long)n_wide, level_first.size(),
-                (unsigned long long)n_records);
+        fprintf(stderr, "[rtb200] wide tree: %llu records on %zu levels (narrow: %llu), blocks of <= %u, packet stack <= %u of %d\n",
+                (unsigned long long)n_wide, level_first.size(), (unsigned long long)n_records, limit, ctx->wide_stack, RT_STACK_SIZE);
     return RT_OK;
 }
 
@@ -988,7 +999,7 @@ int build_bvh_device(RtContext* ctx, int max_depth, int leaf_max)
     cap = std::min({D.c_begin.n, D.c_end.n, D.c_first.n, D.c_info.n, D.c_size.n, D.c_rec.n, D.c_block.n, D.c_nr.n / 7, D.c_fr.n / 7});
     if (int r = reserve_cells(n / 2 + 4096, 0)) return r;
     {
-        const uint32_t root[4] = {0u, n32, 0u, 1u << 6};                        // begin, end, first child, info: a reference cell
+        const uint32_t root[4] = {0u, n32, 0u, 1u << 10};                        // begin, end, first child, info: a reference cell
         RT_CUDA(ctx, cudaMemcpyAsync(D.c_begin.p, &root[0], 4, cudaMemcpyHostToDevice, st));
         RT_CUDA(ctx, cudaMemcpyAsync(D.c_end.p, &root[1], 4, cudaMemcpyHostToDevice, st));
         RT_CUDA(ctx, cudaMemcpyAsync(D.c_info.p, &root[3], 4, cudaMemcpyHostToDevice, st));

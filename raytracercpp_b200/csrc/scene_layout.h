@@ -9,7 +9,7 @@
 //             (pairs, so that the lane that stages a float4 for a 32-ray packet whose rays agree on the sign of a slab's
 //             denominator can swap that pair in place: the packet's slab test then needs no min/max per slab, kernels.cuh;
 //             the three axis slabs are q0 and half of q1)
-//             meta bit 31 = leaf; low 8 bits = number of child records (interior, 1..8); leaf: low 31 bits = triangle count
+//             meta bit 31 = leaf; low 8 bits = number of child records (interior, 1..8; 1..16 in wrecs[]); leaf: low 31 bits = triangle count
 //             meta bit 30 (interior only) = the children block is also in the TOP TABLE, at record offset (meta >> 8) & 0xff
 //             link        = first triangle (leaf) or first child record (interior)
 //             The (<= 8) records of one interior cell are contiguous and start on a 128-byte boundary, so a cell
